@@ -22,6 +22,10 @@ Nested sections: `marginal` (configs[1], marginal-scan GB/s against the HBM roof
 
 --impl reference: the reference's own CPU implementation (oracle/_ref, the unmodified sources) of the same metric:
 compute(computeBoost) on all host cores (one process per core), each step a bounded sample of configs[3]'s shape.
+
+--dump-outputs DIR: after the timed steps, the headline's hit list of its last step (i, j, statistic; every rank's hits
+merged) as DIR/hit_*.npy. The cohort comes from a fixed seed, so two builds run with the same arguments can be compared
+file by file.
 """
 from __future__ import annotations
 
@@ -51,6 +55,24 @@ NCU_TRAFFIC = {
 CPU_MARGINAL_SAMPLE_SNPS = 2_000
 CPU_PAIRWISE_SAMPLE_SNPS = 1_500     # per process and step in the reference arm: 1 124 250 pairs
 CPU_BASELINE_SAMPLE_SNPS = 4_000     # cpu_baseline of the GPU arm (one core, ~15 s): 7 998 000 pairs
+DUMP_BYTES = 64_000_000             # --dump-outputs budget, .npy headers included
+
+
+def dump_outputs(out_dir, columns):
+    """--dump-outputs: equal-length columns of one result as out_dir/<name>.npy in float64, plus row_count.npy (the full
+    length). A result larger than DUMP_BYTES keeps a seeded sample of its rows, in order, and their indices (rows.npy), so
+    that the files of two builds run with the same arguments can be compared one by one."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(next(iter(columns.values())))
+    out = {name: np.asarray(col, np.float64) for name, col in columns.items()}
+    keep = (DUMP_BYTES - 4096) // (8 * (len(out) + 1))
+    if n > keep:
+        rows = np.sort(np.random.default_rng(SEED).choice(n, keep, replace=False))
+        out = {name: col[rows] for name, col in out.items()}
+        out["rows"] = rows.astype(np.float64)
+    out["row_count"] = np.array([n], np.float64)
+    for name, col in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), col)
 
 
 def measured_peaks():
@@ -236,11 +258,12 @@ def pairwise_section(cx: Ctx, shape, K, W, label, headline):
 
     def step():
         n, stats = st.pairwise_scan(30.0, shard=rank, n_shards=world, capacity=cap, hits=d_hits, on_device=True)
+        gathered = None
         if world > 1:   # hit gather over NCCL: counts, then the padded hit buffers (one collective each)
             counts = mg.gather_counts(int(n), world, torch.device("cuda", local))
-            mg.gather_records(d_hits[:max(1, max(counts))], world)
+            gathered = (counts, mg.gather_records(d_hits[:max(1, max(counts))], world))
             n = int(sum(counts))
-        return n, stats
+        return n, stats, gathered
 
     for _ in range(W):
         step()
@@ -250,12 +273,19 @@ def pairwise_section(cx: Ctx, shape, K, W, label, headline):
     ev0.record(cx.stream)
     screen_ms, pairs, cells, n_hits, cand, engine, tiles = [], 0, 0, 0, 0, 0, 0
     for _ in range(K):
-        n_hits, s = step()
+        n_hits, s, gathered = step()
         screen_ms.append(s.screen_ms)
         pairs, cells, cand, engine, tiles = s.pairs_tested, s.word_cells, s.candidates, s.engine, s.tiles
     ev1.record(cx.stream)
     cx.barrier()
     t1, launches = time.perf_counter(), gw.launch_count() - l0
+    if headline and cx.args.dump_outputs and rank == 0:
+        if gathered is None:
+            hits = np.ascontiguousarray(d_hits[:n_hits].cpu().numpy()).view(gw.HIT_DTYPE).reshape(-1)
+        else:
+            counts, recs = gathered
+            hits = mg.merge_hits([mg.tensor_to_hits(recs[r], c) for r, c in enumerate(counts)])
+        dump_outputs(cx.args.dump_outputs, {"hit_i": hits["i"], "hit_j": hits["j"], "hit_stat": hits["stat"]})
     ms_per_step = cx.reduce(ev0.elapsed_time(ev1), "max") / K
     total_pairs = cx.reduce(float(pairs), "sum")
     value = total_pairs / (ms_per_step * 1e-3)
@@ -874,7 +904,9 @@ def reference_arm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed passes of the headline (the nested sections keep their own counts: marginal max(steps, 10), "
+                         "configs[2] min(steps, 10), fixed repetitions elsewhere)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--snps", type=int, default=0, help="marginal section: SNPs (default configs[1])")
@@ -891,7 +923,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ref-procs", type=int, default=0)
     ap.add_argument("--ref-snps", type=int, default=0, help="reference arm: SNPs per process and step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the hit list of the headline's last step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU headline's results; --impl reference has none")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":

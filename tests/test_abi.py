@@ -167,19 +167,3 @@ def test_round2_entry_points_fail_loudly_without_a_device(lib):
     tiles, pairs = gw.shard_schedule(1000, 1, 3, engine=1)
     assert all(I <= J for I, J in tiles) and len(tiles) == (16 * 17 // 2 + 1) // 3
     assert gw.COMPACT_DTYPE.itemsize == 32 and gw.SIG_DTYPE.itemsize == 48
-
-
-def test_binding_library_carries_the_reference_subclass():
-    """oracle/_ref/libgwasref_dev.so (built where /root/reference exists, travels to the GPU box): the reference objects +
-    class DeviceGenotypeTable : public GenoTable + the patched factory, linked against libgwasdev.so."""
-    import subprocess
-    import oracle
-    if not oracle.have_ref_dev():
-        pytest.skip("reference build absent")
-    syms = subprocess.run(["nm", "-DC", oracle.REF_DEV_SO], capture_output=True, text=True).stdout
-    for name in ("DeviceGenotypeTable::selectCaseControl", "DeviceGenotypeTable::getCaseControlContingencyTable",
-                 "DeviceGenotypeTable::getCaseControlGenotypeDistribution", "DeviceGenotypeTable::addGenotypeRow",
-                 "vtable for libgwaspp::genetics::DeviceGenotypeTable"):
-        assert name in syms, name
-    needed = subprocess.run(["readelf", "-d", oracle.REF_DEV_SO], capture_output=True, text=True).stdout
-    assert "libgwasdev.so" in needed
