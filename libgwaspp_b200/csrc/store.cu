@@ -412,6 +412,8 @@ int gwasdev_set_option(gwasdev_store *s, int option, long long value) {
     if (option == GWASDEV_OPT_SCAN_PIECES) GW_REQUIRE(value >= 0 && value <= gwasdev_store::MAX_PIECES, "gwasdev_set_option: 0..%d pieces", gwasdev_store::MAX_PIECES);
     if (option == GWASDEV_OPT_INGEST_CHUNK) GW_REQUIRE(value == 0 || value >= 64, "gwasdev_set_option: ingest chunks of at least 64 bytes");
     GW_REQUIRE(value >= 0, "gwasdev_set_option: negative value");
+    // the tensor-core operand planes and the per-SNP records stored by role follow the plane choice: rebuild them
+    if (option == GWASDEV_OPT_CLASSIC_PLANES && value != s->opt[option]) s->mm_built = s->mma_side_valid = false;
     s->opt[option] = value;
     return GWASDEV_OK;
 }
