@@ -113,6 +113,9 @@ GWASDEV_API int gwasdev_synchronize(gwasdev_store *s);
 #define GWASDEV_OPT_CAND_CAPACITY 8  /* pairwise screen: candidate buffer entries (0 auto); small values exercise the overflow paths */
 #define GWASDEV_OPT_CLASSIC_PLANES 9 /* two-plane tensor-core screen: 0 auto (every SNP puts its two rarest genotype classes on the tensor cores);
                                         1: always the two homozygote planes, as the reference's shortcut counts them */
+#define GWASDEV_OPT_PERM_OPERAND_BYTES 10 /* permutation test: device bytes the SNP-plane operand may keep resident (0 auto: a quarter
+                                             of the device memory); a larger table is expanded and multiplied one SNP chunk at a time (at least
+                                             64 SNPs, the kernel's tile), as is a table whose operand finds the device too full */
 #define GWASDEV_OPT_COUNT 16
 GWASDEV_API int gwasdev_set_option(gwasdev_store *s, int option, long long value);
 
@@ -240,6 +243,47 @@ GWASDEV_API double gwasdev_last_scan_ms(gwasdev_store *s);
  * mode 1: mask-on-the-fly getCaseControlGenotypeDistribution(r, ccs, ccgd) (:609-657), 8 per SNP;
  * mode 2: pre-selected getCaseControlGenotypeDistribution(r, ccgd) (:659-701), 8 per SNP. */
 GWASDEV_API int gwasdev_counts(gwasdev_store *s, uint64_t snp_begin, uint64_t snp_end, int mode, uint32_t *out);
+
+/* ---- label-permutation test of the marginal scan (max(T), PLINK --mperm's EMP1 / EMP2) -------------------------------------- */
+typedef struct {
+    uint64_t n_perm;        /* permutations evaluated by this call */
+    uint64_t snps;          /* SNPs covered */
+    double gemm_ms;         /* device time of the permutation GEMM kernel(s) (CUDA events) */
+    double total_ms;        /* whole call: draws, operands, observed scan, GEMM, reductions */
+    uint32_t planes;        /* operand planes per SNP that were multiplied: 2 (no missing calls in the table) or 3 */
+    uint32_t built_operand; /* 1 when this call expanded the SNP-plane operand (first call, rows changed, or chunked) */
+} gwasdev_perm_stats;
+
+/* Label-permutation test of the current selection over SNPs [snp_begin, snp_end). Permutation first_perm + k makes exactly
+ * n_case of the selection's samples (cases + controls-and-not-cases) cases, drawn as gwasdev_permutation_masks describes, or
+ * takes case_masks[k] (P blocks each) when case_masks != NULL: any non-empty proper subset of the selection (stratified or
+ * family-aware permutations, other traits; the case count may differ between masks). The case genotype counts of every
+ * (SNP, permutation) pair come from one int8 tensor-core GEMM over the samples (permutation case bytes x one-hot SNP planes).
+ * The observed statistics are those of gwasdev_marginal_scan on the same selection. Outputs (each may be NULL; host or device
+ * buffers as on_device), overwritten, not accumulated:
+ *   exceed[2*i + {0,1}]      permutations whose chi2_allelic / chi2_genotypic of SNP snp_begin+i is >= the observed one
+ *   perm_max[3*k + {0,1,2}]  per permutation: max chi2_allelic, max chi2_genotypic over the df-1 (SNP, permutation) elements,
+ *                            the same over the df-2 elements (0 when there are none)
+ *   perm_stats               device buffer only: [n_perm][snp_end - snp_begin] x {chi2_allelic, chi2_genotypic}
+ * Every statistic is bit-identical to gwasdev_marginal_scan's on the permuted selection. Calls over disjoint first_perm ranges
+ * combine by summing exceed and concatenating perm_max. n_perm = 0 is a no-op. */
+GWASDEV_API int gwasdev_marginal_permute(gwasdev_store *s, uint64_t snp_begin, uint64_t snp_end, uint64_t seed,
+                                         uint64_t first_perm, uint64_t n_perm, const uint16_t *case_masks,
+                                         uint32_t *exceed, double *perm_max, double *perm_stats,
+                                         gwasdev_perm_stats *stats, int on_device);
+/* Host arithmetic, no device needed: the case masks (P = gwasdev_plane_blocks(n_samples) blocks each) of permutations
+ * first_perm .. first_perm + n_perm - 1 of the selection (case_mask, ctrl_mask). Selected samples (in either mask; a sample in
+ * both counts once) are walked in increasing position; with `rank` the position inside the selection, `left` the selected
+ * samples not yet visited and `need` the cases still to place, the sample is a case of permutation q iff
+ * ((sim_hash(seed, q, rank) >> 32) * left) >> 32 < need (Knuth's selection sampling; exactly |case_mask| cases). */
+GWASDEV_API int gwasdev_permutation_masks(uint32_t n_samples, const uint16_t *case_mask, const uint16_t *ctrl_mask,
+                                          uint64_t seed, uint64_t first_perm, uint64_t n_perm, uint16_t *out);
+/* Host arithmetic: empirical p-values per SNP and test (emp1 / emp2 [2*i + {0 allelic, 1 genotypic}], each may be NULL) from
+ * the observed statistics and one or more calls' exceed (summed) and perm_max (concatenated) over n_perm permutations:
+ * EMP1 = (exceed + 1) / (n_perm + 1); allelic EMP2 = (1 + #{q : max_a[q] >= chi2_obs}) / (n_perm + 1); genotypic EMP2 compares
+ * p-values, minp_q = min(Q1(max_g1[q]), Q2(max_g2[q])) <= Q_df(chi2_obs), with Q_df the chi-square upper tail; df-0 SNPs get 1. */
+GWASDEV_API int gwasdev_permutation_pvalues(uint64_t n_snps, uint64_t n_perm, const gwasdev_snp_stats *observed,
+                                            const uint32_t *exceed, const double *perm_max, double *emp1, double *emp2);
 
 /* ---- pair tables (K2, per-call virtuals and parity probes) ---------------------------------- */
 /* n pairs (pi[k], pj[k]) -> out[k] = case table[16] then control table[16], 4x4 row-major with the xx

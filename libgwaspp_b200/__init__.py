@@ -35,13 +35,18 @@ assert COMPACT_DTYPE.itemsize == 32 and SIG_DTYPE.itemsize == 48
 
 # gwasdev_set_option keys (include/gwasdev.h)
 OPT_SELECT_KERNEL, OPT_LANES_PER_ROW, OPT_INGEST_CHUNK, OPT_SCAN_PIECES, OPT_MASKED_SCAN, OPT_TRACE, OPT_FOUR_PLANE, \
-    OPT_ROW_TOTALS, OPT_CAND_CAPACITY, OPT_CLASSIC_PLANES = range(10)
+    OPT_ROW_TOTALS, OPT_CAND_CAPACITY, OPT_CLASSIC_PLANES, OPT_PERM_OPERAND_BYTES = range(11)
 
 
 class PairStats(C.Structure):
     _fields_ = [("pairs_tested", C.c_uint64), ("candidates", C.c_uint64), ("hits", C.c_uint64),
                 ("word_cells", C.c_uint64), ("screen_ms", C.c_double), ("total_ms", C.c_double),
                 ("tiles", C.c_uint32), ("tiles_nine_cell", C.c_uint32), ("engine", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class PermStats(C.Structure):
+    _fields_ = [("n_perm", C.c_uint64), ("snps", C.c_uint64), ("gemm_ms", C.c_double), ("total_ms", C.c_double),
+                ("planes", C.c_uint32), ("built_operand", C.c_uint32)]
 
 
 class GwasDevError(RuntimeError):
@@ -64,6 +69,7 @@ ABI_SYMBOLS = [
     "gwasdev_bed_dims", "gwasdev_load_bed", "gwasdev_set_select_mode", "gwasdev_epi_pairs", "gwasdev_create_from_tped",
     "gwasdev_set_option", "gwasdev_set_stream_masks", "gwasdev_marginal_scan_compact", "gwasdev_pairwise_topk",
     "gwasdev_replicate", "gwasdev_pairwise_scan_multi", "gwasdev_shard_schedule", "gwasdev_i8_peak", "gwasdev_l2_read_peak", "gwasdev_gtest_multi", "gwasdev_is_compacted",
+    "gwasdev_marginal_permute", "gwasdev_permutation_masks", "gwasdev_permutation_pvalues",
 ]
 
 
@@ -134,6 +140,9 @@ def load_library():
     L.gwasdev_gtest_multi.argtypes = [C.POINTER(vp), u32, u64, vp, vp, vp, vp]
     L.gwasdev_hbm_read_peak.argtypes = [i32, u64, C.POINTER(C.c_double)]
     L.gwasdev_l2_read_peak.argtypes = [i32, u64, u32, C.POINTER(C.c_double)]
+    L.gwasdev_marginal_permute.argtypes = [vp, u64, u64, u64, u64, u64, vp, vp, vp, vp, C.POINTER(PermStats), i32]
+    L.gwasdev_permutation_masks.argtypes = [u32, vp, vp, u64, u64, u64, vp]
+    L.gwasdev_permutation_pvalues.argtypes = [u64, u64, vp, vp, vp, vp, vp]
     _lib = L
     return L
 
@@ -183,6 +192,33 @@ def simulate_phenotype(seed: int, n_samples: int, n_case: int) -> np.ndarray:
     out = np.zeros(n_samples, np.uint8)
     _check(load_library().gwasdev_simulate_phenotype(seed, n_samples, n_case, _ptr(out)), "gwasdev_simulate_phenotype")
     return out
+
+
+def permutation_masks(n_samples: int, case_mask, ctrl_mask, seed: int, first_perm: int, n_perm: int) -> np.ndarray:
+    """Case masks (n_perm x P uint16 blocks) of permutations first_perm.. of a selection, as gwasdev_marginal_permute draws
+    them on the device (host arithmetic)."""
+    case_mask = np.ascontiguousarray(case_mask, np.uint16)
+    ctrl_mask = np.ascontiguousarray(ctrl_mask, np.uint16)
+    P = plane_blocks(n_samples)
+    assert len(case_mask) == P and len(ctrl_mask) == P
+    out = np.zeros((n_perm, P), np.uint16)
+    _check(load_library().gwasdev_permutation_masks(n_samples, _ptr(case_mask), _ptr(ctrl_mask), seed, first_perm, n_perm, _ptr(out)),
+           "gwasdev_permutation_masks")
+    return out
+
+
+def permutation_pvalues(observed, exceed, perm_max) -> tuple[np.ndarray, np.ndarray]:
+    """EMP1 and EMP2 (max(T)), each (n_snps, 2) = (allelic, genotypic), from the observed statistics (STATS_DTYPE), the summed
+    exceed counts (n_snps, 2) and the concatenated perm_max rows (n_perm, 3) of one or more marginal_permute calls."""
+    observed = np.ascontiguousarray(observed, STATS_DTYPE)
+    exceed = np.ascontiguousarray(exceed, np.uint32).reshape(-1, 2)
+    perm_max = np.ascontiguousarray(perm_max, np.float64).reshape(-1, 3)
+    n = len(observed)
+    assert exceed.shape[0] == n
+    emp1, emp2 = np.zeros((n, 2)), np.zeros((n, 2))
+    _check(load_library().gwasdev_permutation_pvalues(n, perm_max.shape[0], _ptr(observed), _ptr(exceed), _ptr(perm_max),
+                                                      _ptr(emp1), _ptr(emp2)), "gwasdev_permutation_pvalues")
+    return emp1, emp2
 
 
 def pack_row_text_block(line: bytes, n_samples: int, label_state: int = 0):
@@ -457,6 +493,34 @@ class GenoStore:
             out["stats"] = np.zeros(n, STATS_DTYPE)
         _check(self.L.gwasdev_marginal_scan(self.h, snp_begin, snp_end, _ptr(out.get("counts")), _ptr(out.get("mi")),
                                             _ptr(out.get("stats")), 0), "gwasdev_marginal_scan")
+        return out
+
+    def marginal_permute(self, n_perm: int, seed: int = 0, first_perm: int = 0, case_masks=None, snp_begin: int = 0,
+                         snp_end: int | None = None, perm_stats: bool = False):
+        """Label-permutation test of the current selection (gwasdev_marginal_permute): dict with exceed (n_snps, 2),
+        perm_max (n_perm, 3), perm_stats (n_perm, n_snps, 2) when asked for, and stats (PermStats). case_masks: (n_perm, P)
+        uint16 case masks instead of the device draws."""
+        snp_end = self.n_snps if snp_end is None else snp_end
+        n = snp_end - snp_begin
+        if case_masks is not None:
+            case_masks = np.ascontiguousarray(case_masks, np.uint16).reshape(n_perm, self.P)
+        out = {"exceed": np.zeros((n, 2), np.uint32), "perm_max": np.zeros((n_perm, 3), np.float64)}
+        st = PermStats()
+        if perm_stats:
+            import torch
+            dev = torch.empty((n_perm, n, 2), dtype=torch.float64, device=f"cuda:{self.device}")
+            ex = torch.empty((n, 2), dtype=torch.int32, device=dev.device)
+            pm = torch.empty((n_perm, 3), dtype=torch.float64, device=dev.device)
+            _check(self.L.gwasdev_marginal_permute(self.h, snp_begin, snp_end, seed, first_perm, n_perm, _ptr(case_masks),
+                                                   _ptr(ex), _ptr(pm), _ptr(dev), C.byref(st), 1), "gwasdev_marginal_permute")
+            torch.cuda.synchronize(dev.device)
+            out["exceed"], out["perm_max"] = ex.cpu().numpy().view(np.uint32), pm.cpu().numpy()
+            out["perm_stats"] = dev.cpu().numpy()
+        else:
+            _check(self.L.gwasdev_marginal_permute(self.h, snp_begin, snp_end, seed, first_perm, n_perm, _ptr(case_masks),
+                                                   _ptr(out["exceed"]), _ptr(out["perm_max"]), None, C.byref(st), 0),
+                   "gwasdev_marginal_permute")
+        out["stats"] = st
         return out
 
     def marginal_scan_into(self, snp_begin, snp_end, counts=None, mi=None, stats=None, on_device=True):

@@ -194,6 +194,14 @@ struct gwasdev_store {
     std::vector<uint8_t> h_tile_missing;   // host copy of d_tile_missing (valid with side_valid)
     size_t cap_mm = 0, cap_mma_row = 0, cap_mma_col = 0;
     bool mma_side_valid = false;
+    // permutation test (permute.cu): one-hot SNP planes over ALL raw samples, +1 bytes, phenotype-independent -- they survive
+    // re-selection and are dropped by gwasdev_internal_rows_changed
+    bool pb_resident = false;     // d_pb holds the planes of every SNP of the table
+    int pb_missing = -1;          // the table has missing calls (3 planes per SNP) or not (2); -1: not determined yet
+    int8_t *d_pb = nullptr;       // [pb_planes * SNPs][32 * Wr]
+    int8_t *d_pa = nullptr;       // [permutations][32 * Wr]: +1 where the sample is a case of the permutation
+    size_t cap_pb = 0, cap_pa = 0;
+    void *tmap_perm = nullptr;    // host copies of the CUtensorMaps over d_pa and d_pb
     bool any_missing = false, any_clean = false;     // over tiles, valid with side_valid
     bool pc_valid = false;                           // cached pair / tile counts of the last pairwise scan's shard
     int pc_engines = 0;

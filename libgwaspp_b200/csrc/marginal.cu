@@ -112,19 +112,20 @@ __device__ __forceinline__ double maf_reference(const uint32_t ft[4]) {   // alg
     return maf;
 }
 
-__device__ __noinline__ void fill_stats(const uint32_t ca[4], const uint32_t co[4], gwasdev_snp_stats &o) {
-    o.maf_ref_case = maf_reference(ca);
-    o.maf_ref_ctrl = maf_reference(co);
+// The two chi-square statistics of one SNP. Out of line and shared by fill_stats and the permutation test's epilogue
+// (permute_gemm.cuh, compiled in this translation unit), so that both run the same compiled fp64 code: a permuted cohort's
+// statistics are bit-identical to a scan of that cohort.
+struct Chi2 { double allelic, genotypic; int df; };
+__device__ __noinline__ Chi2 chi2_tests(const uint32_t ca[4], const uint32_t co[4]) {
+    Chi2 r;
     const double a_ca = 2.0 * ca[0] + ca[1], b_ca = 2.0 * ca[2] + ca[1];
     const double a_co = 2.0 * co[0] + co[1], b_co = 2.0 * co[2] + co[1];
     const double r1 = a_ca + b_ca, r2 = a_co + b_co, c1 = a_ca + a_co, c2 = b_ca + b_co, t = r1 + r2;
-    o.maf_pooled = t > 0 ? fmin(c1, c2) / t : nan("");
     // allelic 2x2, df 1
-    if (r1 == 0 || r2 == 0 || c1 == 0 || c2 == 0) { o.chi2_allelic = 0.0; o.p_allelic = 1.0; }
+    if (r1 == 0 || r2 == 0 || c1 == 0 || c2 == 0) r.allelic = 0.0;
     else {
         const double d = a_ca * b_co - b_ca * a_co;
-        o.chi2_allelic = t * d * d / (r1 * r2 * c1 * c2);
-        o.p_allelic = chisq_upper(o.chi2_allelic, 1);
+        r.allelic = t * d * d / (r1 * r2 * c1 * c2);
     }
     // genotypic 2x3 Pearson over non-empty genotype columns
     const double g1 = (double)ca[0] + ca[1] + ca[2], g2 = (double)co[0] + co[1] + co[2], gt = g1 + g2;
@@ -140,10 +141,25 @@ __device__ __noinline__ void fill_stats(const uint32_t ca[4], const uint32_t co[
             x += (ca[g] - e1) * (ca[g] - e1) / e1 + (co[g] - e2) * (co[g] - e2) / e2;
         }
     }
-    const int df = cols > 1 ? cols - 1 : 0;
-    o.df_genotypic = df;
-    if (df == 0) { o.chi2_genotypic = 0.0; o.p_genotypic = 1.0; }
-    else { o.chi2_genotypic = x; o.p_genotypic = chisq_upper(x, df); }
+    r.df = cols > 1 ? cols - 1 : 0;
+    r.genotypic = r.df == 0 ? 0.0 : x;
+    return r;
+}
+
+__device__ __noinline__ void fill_stats(const uint32_t ca[4], const uint32_t co[4], gwasdev_snp_stats &o) {
+    o.maf_ref_case = maf_reference(ca);
+    o.maf_ref_ctrl = maf_reference(co);
+    const double a_ca = 2.0 * ca[0] + ca[1], b_ca = 2.0 * ca[2] + ca[1];
+    const double a_co = 2.0 * co[0] + co[1], b_co = 2.0 * co[2] + co[1];
+    const double c1 = a_ca + a_co, c2 = b_ca + b_co, t = (a_ca + b_ca) + (a_co + b_co);
+    o.maf_pooled = t > 0 ? fmin(c1, c2) / t : nan("");
+    const Chi2 x = chi2_tests(ca, co);
+    // chisq_upper(0, df) is 1: the p-value of a degenerate table (statistic 0) as well as of a zero statistic
+    o.chi2_allelic = x.allelic;
+    o.p_allelic = chisq_upper(x.allelic, 1);
+    o.df_genotypic = x.df;
+    o.chi2_genotypic = x.genotypic;
+    o.p_genotypic = chisq_upper(x.genotypic, x.df);
 }
 
 // Where one scan writes. Every pointer may be NULL; outputs are indexed from out_base (the first SNP of the call).
@@ -803,3 +819,7 @@ int gwasdev_counts(gwasdev_store *s, uint64_t snp_begin, uint64_t snp_end, int m
 }
 
 }  // extern "C"
+
+// The permutation test's tensor-core kernel lives in this translation unit so that its epilogue and fill_stats call one
+// compiled chi2_tests.
+#include "permute_gemm.cuh"
