@@ -285,6 +285,55 @@ GWASDEV_API int gwasdev_permutation_masks(uint32_t n_samples, const uint16_t *ca
 GWASDEV_API int gwasdev_permutation_pvalues(uint64_t n_snps, uint64_t n_perm, const gwasdev_snp_stats *observed,
                                             const uint32_t *exceed, const double *perm_max, double *emp1, double *emp2);
 
+/* ---- linkage disequilibrium: genotypic r^2 ----------------------------------------------------------------------------------------
+ * For a sample set S (every sample of the table, or sample_mask: P 16-bit blocks, bit c&15 of block c>>4 for sample c; NULL = all)
+ * and SNPs i, j: x is the allele count under the store's own labels (aa 0, ab 1, bb 2: the {aa, ab, bb} of gwasdev_counts). Over
+ * the samples of S called at both SNPs, the exact integer sums n, Sx, Sy, Sxx, Syy, Sxy give, in int64, num = n Sxy - Sx Sy,
+ * vx = n Sxx - Sx^2, vy = n Syy - Sy^2, and in fp64 without contraction r2 = (num num) / (vx vy), r = num / sqrt(vx vy): the
+ * squared Pearson correlation of allele counts over pairwise-complete samples. Both are NaN when vx = 0 or vy = 0 (a SNP
+ * monomorphic over those samples, n < 2). r2 does not depend on the labels; the sign of r does, and labels are first-seen
+ * (the first homozygote of a row is aa), so r of two SNPs in perfect LD may be -1. Every entry point below computes r and r2
+ * with the same device arithmetic: their values are bit-identical. */
+typedef struct {
+    uint32_t i, j;      /* i < j, table row indices */
+    uint32_t n;         /* samples of S called at both SNPs */
+    uint32_t reserved;
+    double r, r2;
+} gwasdev_ld_pair;      /* 32 bytes */
+typedef struct {
+    uint64_t pairs_tested;   /* pairs (i, j) of the band this call covered */
+    uint64_t pairs_kept;     /* pairs with r2 >= r2_threshold */
+    double gemm_ms;          /* device time of the LD GEMM kernel(s) (CUDA events) */
+    double total_ms;         /* whole call: operand, GEMM, list sort, copies */
+    uint32_t rows_per_snp;   /* operand rows per SNP that were multiplied: 1 (no missing call in S) or 3 */
+    uint32_t built_operand;  /* 1 when this call expanded the operand (first call, rows or sample set changed, or chunked) */
+} gwasdev_ld_stats;
+#define GWASDEV_OPT_LD_OPERAND_BYTES 11 /* LD: device bytes the allele-count operand may keep resident (0 auto: a quarter of the device
+                                           memory); a larger table is expanded one chunk of 256-SNP blocks (plus the window's B-SNPs) at a
+                                           time, as is a table whose operand finds the device too full */
+/* Every pair snp_begin <= i < j < snp_end with j - i <= window (window >= 1; window >= snp_end - snp_begin - 1 is the full LD
+ * matrix of the region), from one int8 tensor-core GEMM of the allele-count rows against themselves restricted to the band.
+ * Works on a freshly loaded table: no selection is needed.
+ *   pairs (may be NULL)  the pairs with r2 >= r2_threshold (fp64 comparison; NaN never qualifies), sorted by (i, j);
+ *                        more than `capacity` of them -> GWASDEV_EOVERFLOW with *n_pairs = the number needed
+ *   band (may be NULL)   (float)r2 at band[(i - snp_begin) * window + (j - i - 1)], NaN where r2 is undefined or j >= snp_end
+ * Host or device buffers as on_device; stats may be NULL. */
+GWASDEV_API int gwasdev_ld_window(gwasdev_store *s, uint64_t snp_begin, uint64_t snp_end, uint32_t window, const uint16_t *sample_mask,
+                                  double r2_threshold, gwasdev_ld_pair *pairs, uint64_t capacity, uint64_t *n_pairs,
+                                  float *band, gwasdev_ld_stats *stats, int on_device);
+/* Given pairs (pi[k], pj[k]) at any distance, i != j in either order -> out[k] with i < j (host buffers). Counts on the CUDA
+ * cores from the raw rows: annotates pair-screen hits and cross-checks the GEMM path. */
+GWASDEV_API int gwasdev_ld_pairs(gwasdev_store *s, uint64_t n, const uint32_t *pi, const uint32_t *pj, const uint16_t *sample_mask,
+                                 gwasdev_ld_pair *out);
+/* Host arithmetic, no device needed: greedy LD pruning of SNPs [snp_begin, snp_end) from a list of gwasdev_ld_window (same
+ * window, threshold at or below r2_threshold; sorted by (i, j), every pair inside the range and the window, else
+ * GWASDEV_EINVAL). Walking i upwards, SNP i is kept (keep[i - snp_begin] = 1) unless some kept k with
+ * max(snp_begin, i - window) <= k < i has r2(k, i) >= r2_threshold. So no two kept SNPs within the window reach the threshold,
+ * and every dropped SNP has a kept SNP before it within the window that does. This is not PLINK's --indep-pairwise: there is
+ * no window step, and the earlier SNP always wins, whatever the allele frequencies. */
+GWASDEV_API int gwasdev_ld_prune(uint64_t snp_begin, uint64_t snp_end, uint32_t window, double r2_threshold,
+                                 const gwasdev_ld_pair *pairs, uint64_t n_pairs, uint8_t *keep);
+
 /* ---- pair tables (K2, per-call virtuals and parity probes) ---------------------------------- */
 /* n pairs (pi[k], pj[k]) -> out[k] = case table[16] then control table[16], 4x4 row-major with the xx
  * row/column (common_genotype.h:182-192).

@@ -30,12 +30,15 @@ COMPACT_DTYPE = np.dtype([("cases", "<u2", 4), ("controls", "<u2", 4), ("chi2_al
                           ("chi2_genotypic", "<f4"), ("p_genotypic", "<f4")])
 SIG_DTYPE = np.dtype([("snp", "<u4"), ("df_genotypic", "<u4"), ("maf_pooled", "<f8"), ("chi2_allelic", "<f8"), ("p_allelic", "<f8"),
                       ("chi2_genotypic", "<f8"), ("p_genotypic", "<f8")])
+# gwasdev_ld_pair: one SNP pair of the LD calls (i < j), its pairwise-complete sample count and genotypic r, r^2
+LD_PAIR_DTYPE = np.dtype([("i", "<u4"), ("j", "<u4"), ("n", "<u4"), ("reserved", "<u4"), ("r", "<f8"), ("r2", "<f8")])
+assert LD_PAIR_DTYPE.itemsize == 32
 assert MI_DTYPE.itemsize == 192 and STATS_DTYPE.itemsize == 64 and HIT_DTYPE.itemsize == 16
 assert COMPACT_DTYPE.itemsize == 32 and SIG_DTYPE.itemsize == 48
 
 # gwasdev_set_option keys (include/gwasdev.h)
 OPT_SELECT_KERNEL, OPT_LANES_PER_ROW, OPT_INGEST_CHUNK, OPT_SCAN_PIECES, OPT_MASKED_SCAN, OPT_TRACE, OPT_FOUR_PLANE, \
-    OPT_ROW_TOTALS, OPT_CAND_CAPACITY, OPT_CLASSIC_PLANES, OPT_PERM_OPERAND_BYTES = range(11)
+    OPT_ROW_TOTALS, OPT_CAND_CAPACITY, OPT_CLASSIC_PLANES, OPT_PERM_OPERAND_BYTES, OPT_LD_OPERAND_BYTES = range(12)
 
 
 class PairStats(C.Structure):
@@ -47,6 +50,11 @@ class PairStats(C.Structure):
 class PermStats(C.Structure):
     _fields_ = [("n_perm", C.c_uint64), ("snps", C.c_uint64), ("gemm_ms", C.c_double), ("total_ms", C.c_double),
                 ("planes", C.c_uint32), ("built_operand", C.c_uint32)]
+
+
+class LdStats(C.Structure):
+    _fields_ = [("pairs_tested", C.c_uint64), ("pairs_kept", C.c_uint64), ("gemm_ms", C.c_double), ("total_ms", C.c_double),
+                ("rows_per_snp", C.c_uint32), ("built_operand", C.c_uint32)]
 
 
 class GwasDevError(RuntimeError):
@@ -70,6 +78,7 @@ ABI_SYMBOLS = [
     "gwasdev_set_option", "gwasdev_set_stream_masks", "gwasdev_marginal_scan_compact", "gwasdev_pairwise_topk",
     "gwasdev_replicate", "gwasdev_pairwise_scan_multi", "gwasdev_shard_schedule", "gwasdev_i8_peak", "gwasdev_l2_read_peak", "gwasdev_gtest_multi", "gwasdev_is_compacted",
     "gwasdev_marginal_permute", "gwasdev_permutation_masks", "gwasdev_permutation_pvalues",
+    "gwasdev_ld_window", "gwasdev_ld_pairs", "gwasdev_ld_prune",
 ]
 
 
@@ -143,6 +152,9 @@ def load_library():
     L.gwasdev_marginal_permute.argtypes = [vp, u64, u64, u64, u64, u64, vp, vp, vp, vp, C.POINTER(PermStats), i32]
     L.gwasdev_permutation_masks.argtypes = [u32, vp, vp, u64, u64, u64, vp]
     L.gwasdev_permutation_pvalues.argtypes = [u64, u64, vp, vp, vp, vp, vp]
+    L.gwasdev_ld_window.argtypes = [vp, u64, u64, u32, vp, C.c_double, vp, u64, C.POINTER(u64), vp, C.POINTER(LdStats), i32]
+    L.gwasdev_ld_pairs.argtypes = [vp, u64, vp, vp, vp, vp]
+    L.gwasdev_ld_prune.argtypes = [u64, u64, u32, C.c_double, vp, u64, vp]
     _lib = L
     return L
 
@@ -219,6 +231,17 @@ def permutation_pvalues(observed, exceed, perm_max) -> tuple[np.ndarray, np.ndar
     _check(load_library().gwasdev_permutation_pvalues(n, perm_max.shape[0], _ptr(observed), _ptr(exceed), _ptr(perm_max),
                                                       _ptr(emp1), _ptr(emp2)), "gwasdev_permutation_pvalues")
     return emp1, emp2
+
+
+def ld_prune(pairs, window: int, r2_threshold: float, snp_begin: int, snp_end: int) -> np.ndarray:
+    """Greedy LD pruning of SNPs [snp_begin, snp_end) (host arithmetic, gwasdev_ld_prune): walking upwards, a SNP is kept unless
+    an earlier kept SNP within `window` has r2 >= r2_threshold with it. pairs: LD_PAIR_DTYPE records sorted by (i, j), as
+    GenoStore.ld_window returns them at a threshold at or below r2_threshold. Returns a bool keep mask over the range."""
+    pairs = np.ascontiguousarray(pairs, LD_PAIR_DTYPE)
+    keep = np.zeros(max(snp_end - snp_begin, 0), np.uint8)
+    _check(load_library().gwasdev_ld_prune(snp_begin, snp_end, window, r2_threshold, _ptr(pairs), len(pairs), _ptr(keep)),
+           "gwasdev_ld_prune")
+    return keep.astype(bool)
 
 
 def pack_row_text_block(line: bytes, n_samples: int, label_state: int = 0):
@@ -564,6 +587,52 @@ class GenoStore:
         out = np.zeros((snp_end - snp_begin, 4 if mode == 0 else 8), np.uint32)
         _check(self.L.gwasdev_counts(self.h, snp_begin, snp_end, mode, _ptr(out)), "gwasdev_counts")
         return out
+
+    # -- linkage disequilibrium
+    def _sample_blocks(self, sample_mask):
+        """None, P uint16 blocks (bit c&15 of block c>>4), or a bool per sample."""
+        if sample_mask is None:
+            return None
+        m = np.asarray(sample_mask)
+        if m.dtype == bool:
+            assert m.shape == (self.n_samples,), m.shape
+            bits = np.zeros(self.P * 16, np.uint8)
+            bits[: self.n_samples] = m
+            return np.packbits(bits, bitorder="little").view(np.uint16).copy()
+        m = np.ascontiguousarray(m, np.uint16)
+        assert m.shape == (self.P,), m.shape
+        return m
+
+    def ld_window(self, window: int, r2_threshold: float = 0.2, snp_begin: int = 0, snp_end: int | None = None, sample_mask=None,
+                  band: bool = False, capacity: int = 1 << 20, pairs: bool = True):
+        """Genotypic r^2 of every pair snp_begin <= i < j < snp_end with j - i <= window (gwasdev_ld_window). Returns (pairs
+        [LD_PAIR_DTYPE] with r2 >= r2_threshold sorted by (i, j), or None; band (n, window) float32 of r2 or None; LdStats).
+        The list grows to the size needed when `capacity` is too small."""
+        snp_end = self.n_snps if snp_end is None else snp_end
+        mask = self._sample_blocks(sample_mask)
+        out = np.zeros(capacity, LD_PAIR_DTYPE) if pairs else None
+        b = np.zeros((max(snp_end - snp_begin, 0), window), np.float32) if band else None
+        st, got = LdStats(), C.c_uint64()
+        rc = self.L.gwasdev_ld_window(self.h, snp_begin, snp_end, window, _ptr(mask), r2_threshold, _ptr(out), capacity if pairs else 0,
+                                      C.byref(got), _ptr(b), C.byref(st), 0)
+        if rc == 4 and pairs:   # GWASDEV_EOVERFLOW: re-run with the size needed
+            return self.ld_window(window, r2_threshold, snp_begin, snp_end, sample_mask, band, int(got.value), pairs)
+        _check(rc, "gwasdev_ld_window")
+        return (out[: got.value].copy() if pairs else None), b, st
+
+    def ld_pairs(self, pi, pj, sample_mask=None) -> np.ndarray:
+        """Genotypic r^2 of given pairs at any distance (i != j, either order): LD_PAIR_DTYPE records with i < j."""
+        pi, pj = self._pairs(pi, pj)
+        out = np.zeros(len(pi), LD_PAIR_DTYPE)
+        _check(self.L.gwasdev_ld_pairs(self.h, len(pi), _ptr(pi), _ptr(pj), _ptr(self._sample_blocks(sample_mask)), _ptr(out)),
+               "gwasdev_ld_pairs")
+        return out
+
+    def ld_prune(self, window: int, r2_threshold: float, snp_begin: int = 0, snp_end: int | None = None, sample_mask=None) -> np.ndarray:
+        """Greedy LD pruning (see ld_prune): ld_window at r2_threshold, then the host rule. Returns a bool keep mask over the range."""
+        snp_end = self.n_snps if snp_end is None else snp_end
+        pairs, _, _ = self.ld_window(window, r2_threshold, snp_begin, snp_end, sample_mask)
+        return ld_prune(pairs, window, r2_threshold, snp_begin, snp_end)
 
     # -- pairs
     def _pairs(self, pi, pj):

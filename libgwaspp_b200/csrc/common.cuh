@@ -202,6 +202,17 @@ struct gwasdev_store {
     int8_t *d_pa = nullptr;       // [permutations][32 * Wr]: +1 where the sample is a case of the permutation
     size_t cap_pb = 0, cap_pa = 0;
     void *tmap_perm = nullptr;    // host copies of the CUtensorMaps over d_pa and d_pb
+    // windowed LD (ld.cu): int8 allele-count operand over the sample set S it was built for -- it survives calls with the same S,
+    // is rebuilt when S changes and is dropped by gwasdev_internal_rows_changed
+    bool ld_sums_valid = false;   // d_ld_sums and ld_missing describe the rows over h_ld_mask
+    bool ld_resident = false;     // d_ld holds the operand of every SNP of the table over h_ld_mask
+    int ld_missing = 0;           // some sample of S has no call at some SNP: three row types per SNP (x, called, x^2), else one (x)
+    std::vector<uint32_t> h_ld_mask;   // S as [Wr] words
+    uint32_t *d_ld_mask = nullptr;     // [Wr]
+    uint2 *d_ld_sums = nullptr;        // [M] (sum x, sum x^2) over S
+    int8_t *d_ld = nullptr;
+    size_t cap_ld = 0;
+    void *tmap_ld = nullptr;      // host copies of the CUtensorMaps over d_ld (A box, B box)
     bool any_missing = false, any_clean = false;     // over tiles, valid with side_valid
     bool pc_valid = false;                           // cached pair / tile counts of the last pairwise scan's shard
     int pc_engines = 0;

@@ -180,6 +180,10 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr) {
 constexpr uint32_t idesc_i8(int n) { return (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(MMA_M >> 4) << 24); }   // M = 256 over the CTA pair
 constexpr uint32_t IDESC_I8 = idesc_i8(MMA_N);
 
+// 2-D tensor map over `rows` operand rows of `kbytes` bytes (K-major, SWIZZLE_128B boxes of 128 bytes x box_rows), as the
+// permutation test and the LD kernel stage them (permute.cu)
+int encode_operand_map(void *ptr, uint64_t rows, uint32_t kbytes, uint32_t box_rows, CUtensorMap *out);
+
 __device__ __forceinline__ uint32_t spread4(uint32_t nibble) { return (nibble * 0x00204081u) & 0x01010101u; }   // bit i -> byte i
 
 }  // namespace gwasdev

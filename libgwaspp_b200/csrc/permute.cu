@@ -112,7 +112,7 @@ static double chisq_q(double x, int df) { return x > 0.0 ? (df == 1 ? std::erfc(
 
 using namespace gwasdev;
 
-static int encode_map(void *ptr, uint64_t rows, uint32_t kbytes, uint32_t box_rows, CUtensorMap *out) {
+int gwasdev::encode_operand_map(void *ptr, uint64_t rows, uint32_t kbytes, uint32_t box_rows, CUtensorMap *out) {
     encode_tiled_fn encode = nullptr;
     { const int rc = get_encode_tiled(&encode); if (rc != GWASDEV_OK) return rc; }
     cuuint64_t gdim[2] = {kbytes, rows};
@@ -121,7 +121,7 @@ static int encode_map(void *ptr, uint64_t rows, uint32_t kbytes, uint32_t box_ro
     cuuint32_t estr[2] = {1, 1};
     const CUresult r = encode(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, ptr, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (permutation operand) failed (%d)", (int)r); return GWASDEV_ENODEVICE; }
+    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (operand rows) failed (%d)", (int)r); return GWASDEV_ENODEVICE; }
     return GWASDEV_OK;
 }
 
@@ -143,8 +143,8 @@ static int launch_perm(gwasdev_store *s, int PL, PermParams p, uint64_t pa_rows,
     const uint32_t kbytes = 32 * s->Wr;
     CUtensorMap *maps = (CUtensorMap *)s->tmap_perm;
     int rc;
-    if ((rc = encode_map(s->d_pa, pa_rows, kbytes, PERM_BLK / 2, &maps[0])) != GWASDEV_OK) return rc;
-    if ((rc = encode_map(s->d_pb, (uint64_t)PL * pb_snps, kbytes, PSNP_HALF * PL, &maps[1])) != GWASDEV_OK) return rc;
+    if ((rc = encode_operand_map(s->d_pa, pa_rows, kbytes, PERM_BLK / 2, &maps[0])) != GWASDEV_OK) return rc;
+    if ((rc = encode_operand_map(s->d_pb, (uint64_t)PL * pb_snps, kbytes, PSNP_HALF * PL, &maps[1])) != GWASDEV_OK) return rc;
     p.NKB = kbytes / MMA_KB;
     p.n_tiles = (uint64_t)p.n_pblk * ((p.nsnp + PSNP_BLK - 1) / PSNP_BLK);
     int sms = 0;

@@ -372,6 +372,7 @@ void gwasdev_internal_rows_changed(gwasdev_store *s) {
     s->tot_valid = false;
     s->pb_resident = false;   // the permutation test's SNP planes depend on the rows only, not on the selection
     s->pb_missing = -1;
+    s->ld_sums_valid = s->ld_resident = false;   // the LD operand depends on the rows and its sample set
 }
 
 extern "C" {
@@ -382,8 +383,8 @@ void gwasdev_destroy(gwasdev_store *s) {
     gwasdev_internal_free_ingest(s);
     cudaFree(s->d_masks); cudaFree(s->d_row_tot); cudaFree(s->d_case_idx); cudaFree(s->d_ctrl_idx);
     cudaFree(s->d_sel); cudaFree(s->d_pw); cudaFree(s->d_mi); cudaFree(s->d_side); cudaFree(s->d_tile_missing);
-    free(s->tmap); free(s->tmap_mm); free(s->tmap_mm4); free(s->tmap_perm);
-    cudaFree(s->d_pa); cudaFree(s->d_pb);
+    free(s->tmap); free(s->tmap_mm); free(s->tmap_mm4); free(s->tmap_perm); free(s->tmap_ld);
+    cudaFree(s->d_pa); cudaFree(s->d_pb); cudaFree(s->d_ld); cudaFree(s->d_ld_mask); cudaFree(s->d_ld_sums);
     cudaFree(s->d_mm); cudaFree(s->d_mm4); cudaFree(s->d_mma_row); cudaFree(s->d_mma_col); cudaFree(s->d_plane_derived); cudaFree(s->d_tile_counter);
     for (gwasdev_store::Scratch *sc : {&s->sc_out_counts, &s->sc_out_stats, &s->sc_out_mi, &s->sc_cnt, &s->sc_cand, &s->sc_keys,
                                       &s->sc_keys2, &s->sc_vals, &s->sc_vals2, &s->sc_sort, &s->sc_hits, &s->sc_pi, &s->sc_pj,
