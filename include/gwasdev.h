@@ -410,8 +410,17 @@ GWASDEV_API int gwasdev_ksa(gwasdev_store *s, uint64_t n, const uint32_t *pi, co
 /* Diagnostic: the screen kernel's fp32 epilogue evaluated on given pairs, to measure its distance from
  * the fp64 statistic (the screen keeps pairs above threshold - margin; see DESIGN.md). */
 GWASDEV_API int gwasdev_ksa_screen_f32(gwasdev_store *s, uint64_t n, const uint32_t *pi, const uint32_t *pj, float *stat);
+/* Diagnostic: the G-test's fp64 division on n operand pairs (host buffers) on `device`. q_fast[k] = the branch-free
+ * division of the IPF sweeps, q_rn[k] = __ddiv_rn(a[k], b[k]), bad[k] = 1 where the fast sequence leaves its range (the
+ * exponent test ptxas applies before its slow path); q_fast has the bits of q_rn wherever bad is 0 and a[k] != 0, and for
+ * a[k] = +0 over a finite, normal b[k]. */
+GWASDEV_API int gwasdev_fp64_div_probe(int device, uint64_t n, const double *a, const double *b, double *q_fast, double *q_rn,
+                                       uint8_t *bad);
 /* computeGTest (epistasis_func.cpp:508-704): exact log-linear G statistic by IPF and the allele-joint
- * log-odds z for n pairs (host buffers). */
+ * log-odds z for n pairs (host buffers). The IPF stops when sum |delta mu| <= 1e-3, as the reference's loop does. On some
+ * sparse tables (e.g. cells absent in one class) that sum settles on a cycle and never gets there, and the reference
+ * loops forever: a fit that has not converged after 1 000 000 sweeps gives stat = NaN. z does not depend on the fit and
+ * is always computed. */
 GWASDEV_API int gwasdev_gtest(gwasdev_store *s, uint64_t n, const uint32_t *pi, const uint32_t *pj, double *stat,
                   double *z);
 /* pairwise_epi_test of src/test/pairwise.c:50-133 on n dense 3x3x2 tables (cs, ct: 9 ints each) and

@@ -78,7 +78,7 @@ ABI_SYMBOLS = [
     "gwasdev_set_option", "gwasdev_set_stream_masks", "gwasdev_marginal_scan_compact", "gwasdev_pairwise_topk",
     "gwasdev_replicate", "gwasdev_pairwise_scan_multi", "gwasdev_shard_schedule", "gwasdev_i8_peak", "gwasdev_l2_read_peak", "gwasdev_gtest_multi", "gwasdev_is_compacted",
     "gwasdev_marginal_permute", "gwasdev_permutation_masks", "gwasdev_permutation_pvalues",
-    "gwasdev_ld_window", "gwasdev_ld_pairs", "gwasdev_ld_prune",
+    "gwasdev_ld_window", "gwasdev_ld_pairs", "gwasdev_ld_prune", "gwasdev_fp64_div_probe",
 ]
 
 
@@ -296,6 +296,19 @@ def pairwise_epi_test(cs, ct, device: int = 0):
     _check(load_library().gwasdev_pairwise_epi_test(device, len(cs), _ptr(cs), _ptr(ct), _ptr(ll), _ptr(p)),
            "gwasdev_pairwise_epi_test")
     return ll, p
+
+
+def fp64_div_probe(a, b, device: int = 0):
+    """The G-test's branch-free fp64 division next to __ddiv_rn on operand arrays a, b (gwasdev_fp64_div_probe):
+    (q_fast, q_rn, bad)."""
+    a = np.ascontiguousarray(a, np.float64).ravel()
+    b = np.ascontiguousarray(b, np.float64).ravel()
+    assert a.shape == b.shape
+    q_fast, q_rn, bad = np.zeros(len(a)), np.zeros(len(a)), np.zeros(len(a), np.uint8)
+    f = load_library().gwasdev_fp64_div_probe
+    f.argtypes = [C.c_int, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    _check(f(device, len(a), _ptr(a), _ptr(b), _ptr(q_fast), _ptr(q_rn), _ptr(bad)), "gwasdev_fp64_div_probe")
+    return q_fast, q_rn, bad.astype(bool)
 
 
 def tped_dims(path: str) -> tuple[int, int]:

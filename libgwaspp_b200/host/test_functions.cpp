@@ -288,7 +288,7 @@ void computeBoost(GeneticData *gd, std::ostream *out) {
     int idx = 0;
     char buf[256];
     for (size_t k = 0; k < passingThreshold.size(); ++k) {
-        if (passingThreshold[k].second > thresholdRecord) {
+        if (passingThreshold[k].second > thresholdRecord) {      // false for NaN: a G-test fit that never converged
             snprintf(buf, sizeof buf, "%7d\t%7d\t%7d\t%f\t%f\t%f\t%f", idx++, (int)passingThreshold[k].first.first,
                      (int)passingThreshold[k].first.second, 0.0, 0.0, passingThreshold[k].second, zval[k]);
             *out << buf << std::endl;

@@ -218,6 +218,15 @@ class Oracle:
                         _p(m1), _p(m2), C.c_uint32(int(n)), C.byref(s), C.byref(z))
         return s.value, z.value
 
+    def gtest_ex(self, ca, co, m1, m2, n):
+        """(stat, z, IPF sweeps, S): go_gtest plus the sweep count and the error scale S of the statistic."""
+        m1 = np.array([m1], MI_DTYPE)
+        m2 = np.array([m2], MI_DTYPE)
+        s, z, sw, S = C.c_double(), C.c_double(), C.c_uint32(), C.c_double()
+        self.L.go_gtest_ex(_p(np.ascontiguousarray(ca, np.uint32)), _p(np.ascontiguousarray(co, np.uint32)),
+                           _p(m1), _p(m2), C.c_uint32(int(n)), C.byref(s), C.byref(z), C.byref(sw), C.byref(S))
+        return s.value, z.value, sw.value, S.value
+
     def pairwise_epi_test(self, cs, ct):
         cs = np.ascontiguousarray(cs, np.int32).reshape(9)
         ct = np.ascontiguousarray(ct, np.int32).reshape(9)

@@ -360,12 +360,20 @@ double go_ksa(const uint32_t ca[16], const uint32_t co[16], const go_marginal_in
  * that mu_ab. = n_ab. while accumulating mu_a.k and mu_.bk, (2) multiply every cell by
  * (n_a.k / mu_a.k)(n_.bk / mu_.bk) using the per-SNP class margins; stop when sum|delta| <= 1e-3.
  * ---------------------------------------------------------------------------------------------- */
-void go_gtest(const uint32_t ca[16], const uint32_t co[16], const go_marginal_information *m1,
-              const go_marginal_information *m2, uint32_t n_individs, double *stat, double *z) {
+/* The reference loops until convergence; on some sparse tables sum |delta| settles on a cycle (the update multiplies by
+ * the row and the column ratio at once) and it never returns. Here, as in gtest_kernel, a fit that has not converged
+ * after GO_IPF_MAX_SWEEPS sweeps gives stat = NaN and reports GO_IPF_MAX_SWEEPS + 1 sweeps; z is computed regardless.
+ * go_gtest_ex also returns the sweeps run and S = sum of |every term added into inter| + |ln tao|, the scale of the
+ * rounding error of the statistic (2n * S * a few ulp). */
+void go_gtest_ex(const uint32_t ca[16], const uint32_t co[16], const go_marginal_information *m1,
+                 const go_marginal_information *m2, uint32_t n_individs, double *stat, double *z, uint32_t *sweeps_out,
+                 double *s_out) {
     double mu[2][9], mu0[2][9], mu_ik[2][3], mu_jk[2][3];
     for (int i = 0; i < 9; ++i) { mu[0][i] = mu[1][i] = 1.0; }
     double err = 18.0;   /* the reference's first error loop never advances its pointers (:551-553) */
-    while (err > 0.001) {
+    uint32_t sweeps = 0;
+    while (err > 0.001 && sweeps <= GO_IPF_MAX_SWEEPS) {
+        ++sweeps;
         memcpy(mu0, mu, sizeof mu);
         memset(mu_ik, 0, sizeof mu_ik);
         memset(mu_jk, 0, sizeof mu_jk);
@@ -394,18 +402,22 @@ void go_gtest(const uint32_t ca[16], const uint32_t co[16], const go_marginal_in
             }
         }
     }
-    double tao = 0.0, inter = 0.0;
+    double tao = 0.0, inter = 0.0, S = 0.0, term;
+#define GO_ADD(x) (term = (x), inter += term, S += fabs(term))
     for (int a = 0; a < 3; ++a)
         for (int b = 0; b < 3; ++b) {
             int i = 3 * a + b;
             double t1, t2;
             uint32_t nca = ca[4 * a + b], nco = co[4 * a + b];
-            if (nca > 0) { t1 = (double)nca / n_individs; inter += t1 * log(t1); } else t1 = 0.0;
-            if (mu[0][i] > 0) { t2 = mu[0][i] / n_individs; inter += -t1 * log(t2); tao += t2; }
-            if (nco > 0) { t1 = (double)nco / n_individs; inter += t1 * log(t1); } else t1 = 0.0;
-            if (mu[1][i] > 0) { t2 = mu[1][i] / n_individs; inter += -t1 * log(t2); tao += t2; }
+            if (nca > 0) { t1 = (double)nca / n_individs; GO_ADD(t1 * log(t1)); } else t1 = 0.0;
+            if (mu[0][i] > 0) { t2 = mu[0][i] / n_individs; GO_ADD(-t1 * log(t2)); tao += t2; }
+            if (nco > 0) { t1 = (double)nco / n_individs; GO_ADD(t1 * log(t1)); } else t1 = 0.0;
+            if (mu[1][i] > 0) { t2 = mu[1][i] / n_individs; GO_ADD(-t1 * log(t2)); tao += t2; }
         }
-    *stat = (inter + log(tao)) * n_individs * 2.0;
+#undef GO_ADD
+    *stat = sweeps > GO_IPF_MAX_SWEEPS ? NAN : (inter + log(tao)) * n_individs * 2.0;
+    if (sweeps_out) *sweeps_out = sweeps;
+    if (s_out) *s_out = S + fabs(log(tao));
 
     /* allele-joint distribution from cells {0,1,2,4,5,6,8,9,10} in 32-bit unsigned arithmetic,
      * products included (:686-700) */
@@ -422,6 +434,11 @@ void go_gtest(const uint32_t ca[16], const uint32_t co[16], const go_marginal_in
     double or_unf = log((double)(d[4] * d[7]) / (double)(d[5] * d[6]));
     double v_unf = 1 / (double)d[4] + 1 / (double)d[5] + 1 / (double)d[6] + 1 / (double)d[7];
     *z = (or_aff - or_unf) / sqrt(v_aff + v_unf);
+}
+
+void go_gtest(const uint32_t ca[16], const uint32_t co[16], const go_marginal_information *m1,
+              const go_marginal_information *m2, uint32_t n_individs, double *stat, double *z) {
+    go_gtest_ex(ca, co, m1, m2, n_individs, stat, z, NULL, NULL);
 }
 
 /* ------------------------------------------------------------------------------------------------

@@ -78,6 +78,12 @@ double go_ksa(const uint32_t ca[16], const uint32_t co[16], const go_marginal_in
 /* ---- a18: exact log-linear G-test by IPF + allele-joint log-odds z (epistasis_func.cpp:508-704) ---- */
 void go_gtest(const uint32_t ca[16], const uint32_t co[16], const go_marginal_information *m1,
               const go_marginal_information *m2, uint32_t n_individs, double *stat, double *z);
+/* The same with the sweep count and the error scale S = sum |terms added into inter| + |ln tao|. A fit that has not
+ * converged after GO_IPF_MAX_SWEEPS sweeps (the reference never returns) gives stat = NaN and GO_IPF_MAX_SWEEPS + 1 sweeps. */
+#define GO_IPF_MAX_SWEEPS 1000000u
+void go_gtest_ex(const uint32_t ca[16], const uint32_t co[16], const go_marginal_information *m1,
+                 const go_marginal_information *m2, uint32_t n_individs, double *stat, double *z, uint32_t *sweeps,
+                 double *s_out);
 /* ---- a19: pairwise_epi_test (src/test/pairwise.c:50-133) and pchisq upper tail (closed forms) ---- */
 double go_pairwise_epi_test(const int cs[9], const int ct[9]);
 double go_chisq_upper(double x, int df);

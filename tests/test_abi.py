@@ -151,6 +151,8 @@ def test_round2_entry_points_fail_loudly_without_a_device(lib):
         gw.i8_peak(0)
     with pytest.raises(gw.GwasDevError):
         gw.l2_read_peak(0)
+    with pytest.raises(gw.GwasDevError, match="no CUDA device"):
+        gw.fp64_div_probe([1.0], [3.0])
     # host arithmetic keeps working without a device: the shard schedule of both engines
     tiles, pairs = gw.shard_schedule(1000, 0, 1, engine=2)
     assert len(tiles) == 8 * 9 // 2 and pairs == 1000 * 999 // 2
