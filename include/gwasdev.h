@@ -194,7 +194,13 @@ GWASDEV_API int gwasdev_select_case_control(gwasdev_store *s, const uint16_t *ca
  * mode 2), the AND+POPC engine, cohorts beyond the packed accumulator with missing calls, or the second marginal scan of a
  * cohort with samples outside both classes. Marginal scans count through the masks on the raw rows (the reference's
  * mask-on-the-fly overload, :609-657: identical counts), and the tensor-core screen, its fp64 re-score and the G-test read
- * raw rows + masks as well. eager != 0 runs K0 inside gwasdev_select_case_control. */
+ * raw rows + masks as well. eager != 0 runs K0 inside gwasdev_select_case_control.
+ * K0 stages one compacted row in 200 KiB of shared memory, so it compacts selections with ceil(n_case / 128) +
+ * ceil(n_ctrl / 128) <= 6 400 (about 819 200 selected samples). Above that, what needs the compacted layout -- eager
+ * selection, the layout probes above and the AND+POPC engine (itself limited to classes below 65 536) -- fails with
+ * GWASDEV_EINVAL, as does the pair screen of such a cohort with missing calls (see gwasdev_set_pair_engine). Marginal scans,
+ * gwasdev_marginal_accumulate, gwasdev_marginal_permute and the pair screen of a table without missing calls never need it
+ * and run up to 2^23 - 1 samples per class. */
 GWASDEV_API int gwasdev_set_select_mode(gwasdev_store *s, int eager);
 /* 1 when the compacted rows of the current selection exist on the device (K0 has run for it), 0 when not, -1 without a selection. */
 GWASDEV_API int gwasdev_is_compacted(const gwasdev_store *s);
@@ -214,7 +220,12 @@ GWASDEV_API int gwasdev_get_selected_rows(gwasdev_store *s, uint64_t first_row, 
  * marginal_information (computeMarginalInformation, genotype/common_genotype_func.cpp:173-219 ==
  * computeMargins, algorithms/epistasis_func.cpp:706-721), MinorAlleleFrequency and the chi-square tests.
  * counts: 8 per SNP = cases{aa,ab,bb,xx}, controls{aa,ab,bb,xx}. Any output pointer may be NULL.
- * on_device = 0: outputs are host buffers (copied back inside the call); 1: device buffers. */
+ * on_device = 0: outputs are host buffers (copied back inside the call); 1: device buffers.
+ * Any selection with classes of up to 2^23 - 1 samples: the class masks are read from shared memory while they fit in
+ * 200 KiB (1 638 400 samples when the classes partition the table, 819 200 otherwise), else from global memory.
+ * p-values: p_allelic = erfc(sqrt(chi2 / 2)), p_genotypic = exp(-chi2 / 2) (df 2) or the erfc form (df 1), 1 at df 0. They
+ * underflow gradually: subnormal below DBL_MIN (chi2 above about 1 409 for df 1, 1 417 for df 2), within two subnormal
+ * steps of the exact tail there, and 0 from about 1 483 (df 1) / 1 490 (df 2). */
 GWASDEV_API int gwasdev_marginal_scan(gwasdev_store *s, uint64_t snp_begin, uint64_t snp_end, uint32_t *counts,
                           gwasdev_marginal_information *mi, gwasdev_snp_stats *stats, int on_device);
 /* The same scan with compact outputs, for callers on the far side of PCIe (select_cc_maf needs the two frequency tables
@@ -385,8 +396,8 @@ GWASDEV_API int gwasdev_gtest_multi(gwasdev_store *const *stores, uint32_t n_sto
  * tiles; 2: tensor cores or GWASDEV_EINVAL. Tile pairs with missing calls (the reference's other branch,
  * compressed_genotype_table5.cpp:1000-1067) take the four-plane tensor-core kernel under the same conditions and the
  * 9-cell AND+POPC kernel otherwise. Cohorts with larger classes (below 2^23 samples each) run on the four-plane kernel
- * with one pair of planes per class (no missing calls) or one accumulator per class (missing calls). Results are
- * identical. */
+ * with one pair of planes per class (no missing calls) or one accumulator per class (missing calls); the latter builds its
+ * operand from the compacted rows and so fails above K0's limit (see gwasdev_set_select_mode). Results are identical. */
 GWASDEV_API int gwasdev_set_pair_engine(gwasdev_store *s, int engine);
 /* Host arithmetic only (works without a device): the tile pairs (I <= J, as SNP-block indices) of the screen's schedule that
  * `shard` of `n_shards` owns, in schedule order, and the pairs i < j < n_snps they cover. engine 2: the tensor-core

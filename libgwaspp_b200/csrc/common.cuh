@@ -243,6 +243,9 @@ struct gwasdev_store {
 void gwasdev_internal_free_ingest(gwasdev_store *s);
 void gwasdev_internal_rows_changed(gwasdev_store *s);      // raw rows were (re)written: everything derived from them is stale (store.cu)
 int gwasdev_internal_ensure_compacted(gwasdev_store *s);   // K0 on demand (store.cu)
+// whether K0 can compact the current selection: its largest form stages one compacted row in 200 KiB of shared memory, so
+// ceil(n_case / 128) + ceil(n_ctrl / 128) <= 6 400 (about 819 200 selected samples)
+inline bool gwasdev_internal_compact_fits(const gwasdev_store *s) { return 2ull * (s->Wc + s->Wt) * sizeof(uint32_t) <= 200 * 1024; }
 
 namespace gwasdev {
 // make sure sc holds at least `bytes`; contents are not preserved

@@ -301,7 +301,9 @@ marginal_scan_kernel(const uint4 *__restrict__ sel, uint32_t stride4, uint32_t Q
 // getCaseControlGenotypeDistribution(rIdx, ccs, ccgd) (compressed_genotype_table5.cpp:609-657), which is all that
 // select_cc_maf, a permutation or another trait over the resident table needs: no K0, no second copy of the table,
 // algorithmic bytes again n_samples / 4 per SNP. A row is [plane 1: Q chunks][plane 2: Q chunks]; the masks (case,
-// control-and-not-case: the compaction's classes) sit in shared memory.
+// control-and-not-case: the compaction's classes) sit in shared memory, or, for cohorts whose masks exceed the shared-memory
+// budget (SMEM_MASK false), are read from global memory through the read-only path, where every warp of the grid hits the
+// same L2 lines.
 __device__ __forceinline__ void accumulate_masked(const uint4 &x, const uint4 &y, const uint4 &m, HS &h1, HS &h2, HS &hb) {
     const uint4 xm = make_uint4(x.x & m.x, x.y & m.y, x.z & m.z, x.w & m.w);
     const uint4 ym = make_uint4(y.x & m.x, y.y & m.y, y.z & m.z, y.w & m.w);
@@ -318,14 +320,16 @@ __device__ __forceinline__ void accumulate_masked(const uint4 &x, const uint4 &y
 // MODE 2 (partition, totals cached): three masked streams; the row totals come from row_tot (16 bytes per SNP instead of
 //         a second pass over the words). This is what every re-selection over a resident table runs: the ALU work of the
 //         compacted scan plus the mask ANDs, without K0 ever having run.
-template <int G, int SLOTS, int MINB, int MODE>
+template <int G, int SLOTS, int MINB, int MODE, bool SMEM_MASK = true>
 __global__ void __launch_bounds__(256, MINB)
 marginal_scan_masked_kernel(const uint4 *__restrict__ raw, uint32_t Q, const uint4 *__restrict__ mask_case,
                             const uint4 *__restrict__ mask_ctrl, uint32_t n_case, uint32_t n_ctrl, uint64_t snp_begin,
                             uint64_t snp_end, const __grid_constant__ ScanOut out) {
     extern __shared__ uint4 sm_mask[];   // [Q] case, then (MODE 0) [Q] control
-    for (uint32_t q = threadIdx.x; q < (MODE == 0 ? 2 * Q : Q); q += blockDim.x) sm_mask[q] = q < Q ? mask_case[q] : mask_ctrl[q - Q];
-    __syncthreads();
+    if (SMEM_MASK) {
+        for (uint32_t q = threadIdx.x; q < (MODE == 0 ? 2 * Q : Q); q += blockDim.x) sm_mask[q] = q < Q ? mask_case[q] : mask_ctrl[q - Q];
+        __syncthreads();
+    }
     const uint32_t lane = threadIdx.x & 31, g = lane / G, l = lane % G;
     const uint32_t group_mask = G == 32 ? 0xffffffffu : (((1u << G) - 1u) << (g * G));
     constexpr uint32_t NG = 32 / G;
@@ -357,9 +361,9 @@ marginal_scan_masked_kernel(const uint4 *__restrict__ raw, uint32_t Q, const uin
                 for (int u = 0; u < SLOTS; ++u) {
                     const uint32_t q = q0 + u * G;
                     if (q < Q) {
-                        accumulate_masked(x[u], y[u], sm_mask[q], a1, a2, ab);
+                        accumulate_masked(x[u], y[u], SMEM_MASK ? sm_mask[q] : __ldg(mask_case + q), a1, a2, ab);
                         if (MODE == 1) { ChunkPair c; c.x = x[u]; c.y = y[u]; accumulate_pair(c, b1, b2, bb); }   // row totals (bits beyond sample N are zero)
-                        else if (MODE == 0) accumulate_masked(x[u], y[u], sm_mask[Q + q], b1, b2, bb);
+                        else if (MODE == 0) accumulate_masked(x[u], y[u], SMEM_MASK ? sm_mask[Q + q] : __ldg(mask_ctrl + q), b1, b2, bb);
                     }
                 }
             }
@@ -490,7 +494,7 @@ static int scan_compacted(gwasdev_store *s, uint64_t snp_begin, uint64_t snp_end
 
 static size_t masked_smem_bytes(const gwasdev_store *s, int mode) { return (mode == 0 ? 2ull : 1ull) * (s->Wr / 4) * sizeof(uint4); }
 static bool partitioned(const gwasdev_store *s) { return s->n_case + s->n_ctrl == s->N; }   // nobody outside the two classes
-// can this selection be scanned through the masks (the masks must fit in shared memory)
+// do the masks of this selection fit in shared memory
 static bool masked_fits(const gwasdev_store *s) { return masked_smem_bytes(s, partitioned(s) ? 1 : 0) <= 200 * 1024; }
 
 // The masked scan over the raw rows (no compacted store needed).
@@ -512,15 +516,18 @@ static int scan_masked(gwasdev_store *s, uint64_t snp_begin, uint64_t snp_end, S
     if (const char *cfg = getenv("GWASDEV_MSCAN_CFG")) sscanf(cfg, "%d,%d,%d", &slots, &minb, &G);
 #endif
     const uint64_t n = snp_end - snp_begin;
-    const size_t smem = masked_smem_bytes(s, mode);
-    GW_REQUIRE(smem <= 200 * 1024, "masked scan: %u samples exceed the shared-memory mask buffer", s->N);
+    const bool in_smem = masked_smem_bytes(s, mode) <= 200 * 1024;   // else the kernel reads the masks from global memory
+    const size_t smem = in_smem ? masked_smem_bytes(s, mode) : 0;
     const unsigned blocks = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)sms * minb, (n + 255) / 256));
     const uint4 *raw = reinterpret_cast<const uint4 *>(s->d_raw);
     const uint4 *mca = reinterpret_cast<const uint4 *>(s->d_case_sel_mask), *mco = reinterpret_cast<const uint4 *>(s->d_ctrl_sel_mask);
 #define MSCAN1(GG, SS, BB, MM)                                                                                                     \
     do {                                                                                                                           \
-        if (smem > 48 * 1024) GW_CUDA(cudaFuncSetAttribute(marginal_scan_masked_kernel<GG, SS, BB, MM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        marginal_scan_masked_kernel<GG, SS, BB, MM><<<blocks, 256, smem, s->stream>>>(raw, Q, mca, mco, s->n_case, s->n_ctrl, snp_begin, snp_end, out); \
+        if (!in_smem) marginal_scan_masked_kernel<GG, SS, BB, MM, false><<<blocks, 256, 0, s->stream>>>(raw, Q, mca, mco, s->n_case, s->n_ctrl, snp_begin, snp_end, out); \
+        else {                                                                                                                     \
+            if (smem > 48 * 1024) GW_CUDA(cudaFuncSetAttribute(marginal_scan_masked_kernel<GG, SS, BB, MM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+            marginal_scan_masked_kernel<GG, SS, BB, MM><<<blocks, 256, smem, s->stream>>>(raw, Q, mca, mco, s->n_case, s->n_ctrl, snp_begin, snp_end, out); \
+        }                                                                                                                          \
     } while (0)
 #define MSCAN(GG, SS, BB)                                                                                                          \
     do { if (mode == 2) MSCAN1(GG, SS, BB, 2); else if (mode == 1) MSCAN1(GG, SS, BB, 1); else MSCAN1(GG, SS, BB, 0); } while (0)
@@ -557,9 +564,12 @@ static int scan_masked(gwasdev_store *s, uint64_t snp_begin, uint64_t snp_end, S
 // Which kernel a marginal scan runs: the compacted layout when it exists; otherwise through the masks on the raw rows
 // (no K0) -- always when the classes partition the cohort (with cached row totals that costs what the compacted scan
 // costs), else for the first scan after a selection only: the second builds the compacted layout, which every later
-// scan streams with half the popcount work per byte.
+// scan streams with half the popcount work per byte. A selection K0 cannot compact (gwasdev_internal_compact_fits) is
+// always scanned through the masks, from global memory when they do not fit in shared memory.
 static bool choose_masked(gwasdev_store *s) {
-    if (s->sel_built || s->opt[GWASDEV_OPT_MASKED_SCAN] != 0 || !masked_fits(s)) return false;
+    if (s->sel_built) return false;
+    if (!gwasdev_internal_compact_fits(s)) return true;
+    if (s->opt[GWASDEV_OPT_MASKED_SCAN] != 0 || !masked_fits(s)) return false;
     return partitioned(s) || s->scans_since_select == 0;
 }
 

@@ -734,6 +734,8 @@ int gwasdev_get_selected_rows(gwasdev_store *s, uint64_t first_row, uint64_t n_r
 int gwasdev_internal_ensure_compacted(gwasdev_store *s) {
     GW_REQUIRE(s->selected, "call gwasdev_select_case_control first");
     if (s->sel_built) return GWASDEV_OK;
+    GW_REQUIRE(gwasdev_internal_compact_fits(s), "compacted layout: %u selected samples exceed the compaction kernel's row buffer "
+               "(about 819 200; scans, screens and permutations need no compacted layout)", s->n_case + s->n_ctrl);
     GW_CUDA(cudaSetDevice(s->device));
     const uint32_t stride = 2 * (s->Wc + s->Wt);
     GW_CUDA(reserve_raw(s->d_sel, s->cap_sel, s->M * (uint64_t)stride * 4));
@@ -774,7 +776,6 @@ int gwasdev_internal_ensure_compacted(gwasdev_store *s) {
         const unsigned grid = (unsigned)std::min<uint64_t>((s->M + SNPS - 1) / SNPS, (uint64_t)sms * per_sm);
         select_kernel<true, SNPS><<<grid, 256, smem, s->stream>>>(s->d_raw, s->Wr, ta, to, s->d_sel, stride, s->Wc, s->Wt, s->M);
     } else {
-        GW_REQUIRE(smem_rows / SNPS <= 200 * 1024, "gwasdev_select_case_control: %u samples exceed the compaction kernel's row buffer", s->N);
         GW_CUDA(cudaFuncSetAttribute(select_kernel<false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem_rows / SNPS)));
         const unsigned grid = (unsigned)std::min<uint64_t>(s->M, (uint64_t)sms * 4);
         select_kernel<false, 1><<<grid, 256, smem_rows / SNPS, s->stream>>>(s->d_raw, s->Wr, ta, to, s->d_sel, stride, s->Wc, s->Wt, s->M);
