@@ -375,6 +375,37 @@ GWASDEV_API int gwasdev_pairwise_scan(gwasdev_store *s, double threshold, uint32
  * top_k of their union is the global answer (gwasdev_pairwise_scan_multi does that). */
 GWASDEV_API int gwasdev_pairwise_topk(gwasdev_store *s, double threshold, uint64_t top_k, uint32_t shard, uint32_t n_shards,
                           gwasdev_hit *hits, uint64_t *n_hits, gwasdev_pair_stats *stats, int on_device);
+/* ---- pair screens over chosen SNP sets ---------------------------------------------------------------------------------------
+ * computeBoost's pre-screen restricted to the pairs a study asks for: every unordered pair {i, j}, i != j, with i in A and j in B,
+ * each once. set_b == NULL means B = A (every pair within A); B = all SNPs is set-by-all (PLINK --epistasis set-by-all); two gene
+ * lists give set-by-set. Both sets are strictly increasing SNP indices below the table's SNP count, else GWASDEV_EINVAL (n_b is
+ * ignored when set_b == NULL); a set without pairs (an empty set, A = B of one SNP) gives 0 hits.
+ * Records are gwasdev_hit in table indices, i < j, sorted by (i, j). top_k == 0: every pair whose statistic exceeds the threshold,
+ * capacity and GWASDEV_EOVERFLOW as for gwasdev_pairwise_scan; top_k != 0: gwasdev_pairwise_topk's result (ties at the k-th place
+ * go to the smaller (i, j) in table indices). Every record has the bits of the whole-table screen's record of that pair: the result
+ * is the whole-table hit list filtered to the wanted pairs (for top_k, the top_k of that filtered list).
+ * How: the rows of A u B are gathered into a sub-table on the same device (rows C = A n B, then A \ B, then B \ A, each in table
+ * order), which takes this store's options, engine and selection, builds its own margins and operands -- memory of a table of
+ * |A u B| SNPs, freed when the call returns -- and runs the tensor-core screens over the tiles of its schedule that hold a wanted
+ * pair (gwasdev_set_schedule). Shards (shard / n_shards) partition that tile list as the whole-table calls partition theirs; the
+ * union of the shards' hits is the unsharded result. stats: pairs_tested = wanted pairs of the shard (summed over the shards:
+ * |A| |B| - |C| - |C| (|C| - 1) / 2 with C = A n B), screen_ms = the screen kernels, total_ms = the whole call including the
+ * gather and the operand build. Set screens run on the tensor-core engines only: with gwasdev_set_pair_engine(s, 1), or a selection
+ * whose tiles would go to the AND+POPC kernels, the call returns GWASDEV_EINVAL. Requires gwasdev_select_case_control. */
+GWASDEV_API int gwasdev_pairwise_scan_sets(gwasdev_store *s, const uint32_t *set_a, uint64_t n_a, const uint32_t *set_b, uint64_t n_b,
+                                           double threshold, uint64_t top_k, uint32_t shard, uint32_t n_shards,
+                                           gwasdev_hit *hits, uint64_t capacity, uint64_t *n_hits, gwasdev_pair_stats *stats, int on_device);
+/* Host arithmetic only (works without a device): the set screen's own tile enumeration for sets of a table of n_snps SNPs and
+ * n_samples individuals. With c1 = |C| and a1 = |C| + |A \ B|, sub-table pair gi < gj is wanted when gi < c1, or c1 <= gi < a1 <= gj.
+ * tile_snps 128: the two-plane kernel's tiles, 64: the four-plane kernel's (its modes 0 and 1; the two-accumulator mode bands its
+ * class-padded rows). Listed are the tiles (I <= J, SNP-block indices of the sub-table) of the tensor-core schedule of the sub-table
+ * (gwasdev_shard_schedule, engine 2) that hold at least one wanted pair, in schedule order; `shard` owns list positions p with
+ * (p / 64) % n_shards == shard. tiles (may be NULL) receives min(*n_tiles, capacity) (I, J) pairs; *n_pairs = the wanted pairs
+ * they hold. Input checks as for gwasdev_pairwise_scan_sets. */
+GWASDEV_API int gwasdev_set_schedule(uint64_t n_snps, uint64_t n_samples, uint32_t tile_snps, const uint32_t *set_a, uint64_t n_a,
+                                     const uint32_t *set_b, uint64_t n_b, uint32_t shard, uint32_t n_shards, uint32_t *tiles,
+                                     uint64_t capacity, uint64_t *n_tiles, uint64_t *n_pairs);
+
 /* ---- several devices, one host process (the multi-GPU driver a C++ caller reaches) -------------------------------------
  * Copy of a store on another device: headers and raw rows travel device to device (NVLink when peer access is available),
  * options, engine choice and the current selection are re-applied. What a caller does after loading the genotype file once. */

@@ -79,6 +79,7 @@ ABI_SYMBOLS = [
     "gwasdev_replicate", "gwasdev_pairwise_scan_multi", "gwasdev_shard_schedule", "gwasdev_i8_peak", "gwasdev_l2_read_peak", "gwasdev_gtest_multi", "gwasdev_is_compacted",
     "gwasdev_marginal_permute", "gwasdev_permutation_masks", "gwasdev_permutation_pvalues",
     "gwasdev_ld_window", "gwasdev_ld_pairs", "gwasdev_ld_prune", "gwasdev_fp64_div_probe",
+    "gwasdev_pairwise_scan_sets", "gwasdev_set_schedule",
 ]
 
 
@@ -124,6 +125,9 @@ def load_library():
     L.gwasdev_replicate.argtypes = [vp, i32, C.POINTER(vp)]
     L.gwasdev_pairwise_scan_multi.argtypes = [C.POINTER(vp), u32, C.c_double, u64, vp, u64, C.POINTER(u64), C.POINTER(PairStats), i32]
     L.gwasdev_shard_schedule.argtypes = [u64, u64, i32, u32, u32, vp, u64, C.POINTER(u64), C.POINTER(u64)]
+    L.gwasdev_pairwise_scan_sets.argtypes = [vp, vp, u64, vp, u64, C.c_double, u64, u32, u32, vp, u64, C.POINTER(u64),
+                                             C.POINTER(PairStats), i32]
+    L.gwasdev_set_schedule.argtypes = [u64, u64, u32, vp, u64, vp, u64, u32, u32, vp, u64, C.POINTER(u64), C.POINTER(u64)]
     L.gwasdev_ksa.argtypes = [vp, u64, vp, vp, vp]
     L.gwasdev_ksa_screen_f32.argtypes = [vp, u64, vp, vp, vp]
     L.gwasdev_gtest.argtypes = [vp, u64, vp, vp, vp, vp]
@@ -348,6 +352,34 @@ def shard_schedule(n_snps: int, shard: int, n_shards: int, engine: int = 2, n_sa
     _check(L.gwasdev_shard_schedule(n_snps, n_samples, engine, shard, n_shards, None, 0, C.byref(nt), C.byref(npairs)), "gwasdev_shard_schedule")
     tiles = np.zeros((nt.value, 2), np.uint32)
     _check(L.gwasdev_shard_schedule(n_snps, n_samples, engine, shard, n_shards, _ptr(tiles), nt.value, C.byref(nt), C.byref(npairs)), "gwasdev_shard_schedule")
+    return tiles, int(npairs.value)
+
+
+def _snp_set(x, n_snps: int):
+    """SNP index array or bool mask over the table -> uint32 indices (the library checks order and range)."""
+    a = np.asarray(x)
+    if a.dtype == np.bool_:
+        if a.shape != (n_snps,):
+            raise GwasDevError(f"a SNP mask must have one entry per SNP ({n_snps}), got shape {a.shape}")
+        return np.flatnonzero(a).astype(np.uint32)
+    if a.size and (not np.issubdtype(a.dtype, np.integer) or a.min() < 0 or a.max() >= 1 << 32):
+        raise GwasDevError("SNP sets are non-negative integer indices or bool masks")
+    return np.ascontiguousarray(a, np.uint32).ravel()
+
+
+def set_schedule(n_snps: int, a, b=None, shard: int = 0, n_shards: int = 1, tile_snps: int = 128, n_samples: int = 10_000):
+    """Tiles ((I, J) SNP-block indices of the gathered sub-table, [n, 2]) the shard owns in the set screen of sets a and b
+    (b=None: every pair within a), and the wanted pairs they hold: the library's own enumeration (host arithmetic, no device
+    needed). tile_snps 128: the two-plane kernel's tiles, 64: the four-plane kernel's."""
+    L = load_library()
+    a = _snp_set(a, n_snps)
+    b = None if b is None else _snp_set(b, n_snps)
+    nb = 0 if b is None else len(b)
+    nt, npairs = C.c_uint64(), C.c_uint64()
+    args = (n_snps, n_samples, tile_snps, _ptr(a), len(a), _ptr(b), nb, shard, n_shards)
+    _check(L.gwasdev_set_schedule(*args, None, 0, C.byref(nt), C.byref(npairs)), "gwasdev_set_schedule")
+    tiles = np.zeros((nt.value, 2), np.uint32)
+    _check(L.gwasdev_set_schedule(*args, _ptr(tiles), nt.value, C.byref(nt), C.byref(npairs)), "gwasdev_set_schedule")
     return tiles, int(npairs.value)
 
 
@@ -723,6 +755,24 @@ class GenoStore:
         other.n_snps, other.n_samples, other.device, other.P = self.n_snps, self.n_samples, device, self.P
         other.n_case, other.n_ctrl = self.n_case, self.n_ctrl
         return other
+
+    def pairwise_scan_sets(self, a, b=None, threshold: float = 30.0, top_k: int = 0, shard: int = 0, n_shards: int = 1,
+                           capacity: int = 1 << 20):
+        """The pair screen over every pair {i in a, j in b}, i != j (b=None: every pair within a). a and b are SNP index arrays
+        (strictly increasing) or bool masks over the table, e.g. ld_prune's keep mask. Returns (hits[HIT_DTYPE] in table indices
+        sorted by (i, j), PairStats); top_k != 0 keeps the top_k largest statistics as pairwise_topk does."""
+        a = _snp_set(a, self.n_snps)
+        b = None if b is None else _snp_set(b, self.n_snps)
+        cap = top_k if top_k else capacity
+        hits = np.zeros(max(cap, 1), HIT_DTYPE)
+        st = PairStats()
+        n = C.c_uint64()
+        rc = self.L.gwasdev_pairwise_scan_sets(self.h, _ptr(a), len(a), _ptr(b), 0 if b is None else len(b), threshold, top_k, shard,
+                                               n_shards, _ptr(hits), cap, C.byref(n), C.byref(st), 0)
+        if rc == 4 and not top_k:   # GWASDEV_EOVERFLOW: grow and retry once
+            return self.pairwise_scan_sets(a, b, threshold, 0, shard, n_shards, int(n.value))
+        _check(rc, "gwasdev_pairwise_scan_sets")
+        return hits[: n.value].copy(), st
 
     def pairwise_scan(self, threshold: float = 30.0, shard: int = 0, n_shards: int = 1, capacity: int = 1 << 20,
                       hits=None, on_device: bool = False):

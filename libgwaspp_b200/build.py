@@ -12,7 +12,7 @@ LIB = os.path.join(HERE, "libgwasdev.so")
 SWEEP_LIB = os.path.join(HERE, "libgwasdev_sweep.so")
 HOST_LIB = os.path.join(HERE, "libgwaspp_host.so")
 HOST_CLI = os.path.join(HERE, "gwas_b200")
-SOURCES = ["store.cu", "ingest.cu", "marginal.cu", "pairwise.cu", "pairwise_mma.cu", "multi_device.cu", "permute.cu", "ld.cu"]
+SOURCES = ["store.cu", "ingest.cu", "marginal.cu", "pairwise.cu", "pairwise_mma.cu", "multi_device.cu", "permute.cu", "ld.cu", "pair_sets.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr", "-I", os.path.join(ROOT, "include")]
 

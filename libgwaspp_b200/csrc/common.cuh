@@ -214,6 +214,9 @@ struct gwasdev_store {
     size_t cap_ld = 0;
     void *tmap_ld = nullptr;      // host copies of the CUtensorMaps over d_ld (A box, B box)
     bool any_missing = false, any_clean = false;     // over tiles, valid with side_valid
+    // gathered sub-table of a set screen (pair_sets.cu): per row, its table index | (1 << 31) when one of its genotype classes aa,
+    // ab, bb is empty. Its per-SNP records then leave such a class out of the statistic instead of making it NaN (see set_pair_live)
+    uint32_t *d_set_keys = nullptr;
     bool pc_valid = false;                           // cached pair / tile counts of the last pairwise scan's shard
     int pc_engines = 0;
     uint32_t pc_shard = 0, pc_n_shards = 0;
@@ -243,6 +246,9 @@ struct gwasdev_store {
 void gwasdev_internal_free_ingest(gwasdev_store *s);
 void gwasdev_internal_rows_changed(gwasdev_store *s);      // raw rows were (re)written: everything derived from them is stale (store.cu)
 int gwasdev_internal_ensure_compacted(gwasdev_store *s);   // K0 on demand (store.cu)
+// options, pair engine, selection mode and the current selection of src applied to dst, a store over the same samples: what
+// gwasdev_replicate and the set screens' gathered sub-tables carry over from the store they copy (store.cu)
+int gwasdev_internal_replay_settings(const gwasdev_store *src, gwasdev_store *dst);
 // whether K0 can compact the current selection: its largest form stages one compacted row in 200 KiB of shared memory, so
 // ceil(n_case / 128) + ceil(n_ctrl / 128) <= 6 400 (about 819 200 selected samples)
 inline bool gwasdev_internal_compact_fits(const gwasdev_store *s) { return 2ull * (s->Wc + s->Wt) * sizeof(uint32_t) <= 200 * 1024; }

@@ -94,14 +94,7 @@ int gwasdev_replicate(gwasdev_store *src, int device, gwasdev_store **out) {
     cudaError_t e = cudaMemcpyPeer(dst->d_hdr, device, src->d_hdr, src->device, src->M * sizeof(uint16_t));
     if (e == cudaSuccess) e = cudaMemcpyPeer(dst->d_raw, device, src->d_raw, src->device, src->M * 2ull * src->Wr * sizeof(uint32_t));
     if (e != cudaSuccess) { set_error("gwasdev_replicate: %s", cudaGetErrorString(e)); gwasdev_destroy(dst); return GWASDEV_ENODEVICE; }
-    for (int o = 0; o < GWASDEV_OPT_COUNT; ++o) dst->opt[o] = src->opt[o];
-    dst->pair_engine = src->pair_engine;
-    dst->eager_select = src->eager_select;
-    if (src->selected && !src->h_given_masks.empty()) {
-        const uint16_t *m = src->h_given_masks.data();
-        rc = gwasdev_select_case_control(dst, m, m + src->P);
-        if (rc != GWASDEV_OK) { gwasdev_destroy(dst); return rc; }
-    }
+    if ((rc = gwasdev_internal_replay_settings(src, dst)) != GWASDEV_OK) { gwasdev_destroy(dst); return rc; }
     *out = dst;
     return GWASDEV_OK;
 }

@@ -46,6 +46,12 @@ struct CandSink {
     unsigned long long raise_from, raise_mask;   // raise when slot + 1 >= raise_from and ((slot + 1) & raise_mask) == 0
 };
 
+// One launch of a set screen (pair_sets.cu): the shard's tiles (I2, J) of that kernel's block size in device memory, and the
+// segment bounds c1, a1 of the gathered sub-table (set_pair_wanted in pairwise_mma.cu)
+struct SetLaunch { const uint2 *tiles; uint64_t n_tiles; uint64_t c1, a1; };
+// A set screen on a gathered sub-table: its segment bounds and, on the device, the table row of every sub-table row
+struct SetScreen { uint64_t c1, a1; const uint32_t *d_map; };
+
 // threshold the pairs of the next tile are tested against
 __device__ __forceinline__ float sink_threshold(const CandSink &s) {
     if (!s.hist) return s.thr;

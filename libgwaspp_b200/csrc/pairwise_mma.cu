@@ -35,6 +35,8 @@
 #include "mma_common.cuh"
 
 int gwasdev_internal_ensure_side(gwasdev_store *s);   // pairwise.cu: margins, PairSide records, missing-call flags
+int gwasdev_internal_set_rows(uint64_t M, const uint32_t *set_a, uint64_t n_a, const uint32_t *set_b, uint64_t n_b, const char *who,
+                              std::vector<uint32_t> &map, uint64_t *c1, uint64_t *a1);   // pair_sets.cu
 
 namespace gwasdev {
 
@@ -90,6 +92,10 @@ struct MmaParams {
     uint32_t dump_rank;
     unsigned long long *prof;   // role timers (builds with -DGWASDEV_SWEEP only, GWASDEV_MMA_PROF): per CTA {mma busy, mma waiting for tempty,
                                 // mma waiting for full, epilogue busy, epilogue waiting for tfull, producer waiting for empty, tiles} in SM clocks
+    // set screens (SETS instantiations only; appended so that the fields above keep their offsets): the shard's tiles as
+    // (I2, J), n_tiles of them, and the segment bounds of the gathered sub-table (set_pair_wanted)
+    const uint2 *set_tiles;
+    uint64_t set_c1, set_a1;
 };
 #ifdef GWASDEV_SWEEP
 #define GW_PROF(x) x
@@ -125,6 +131,22 @@ __host__ __device__ inline uint64_t shard_tiles_before(uint64_t n, uint32_t shar
     uint64_t cnt = (chunk / n_shards) * SHARD_CHUNK + (chunk % n_shards > shard ? SHARD_CHUNK : 0);
     if (chunk % n_shards == shard) cnt += rem;
     return cnt;
+}
+
+// Set screens run on a gathered sub-table whose rows are C = A n B, then A \ B, then B \ A (each in table order), with
+// c1 = |C| and a1 = |C| + |A \ B|. Pair gi < gj of the sub-table is wanted when gi lies in C, or gi in A \ B and gj in
+// B \ A: every unordered pair {i in A, j in B, i != j} exactly once.
+__host__ __device__ __forceinline__ bool set_pair_wanted(uint64_t gi, uint64_t gj, uint64_t c1, uint64_t a1) {
+    return (gi < c1) | ((gi < a1) & (gj >= a1));
+}
+// Across segments the sub-table may hold a pair in the other order than the table. The statistic is symmetric in the two SNPs
+// except where one of them has an empty genotype class: it is NaN when that is the SNP with the larger table index (0 / 0 in
+// ksa_f64) and finite otherwise. So the sub-table's records leave empty classes out (SETS in mma_side_kernel, pair_side_kernel),
+// every pair evaluates finite, and the pairs whose statistic is NaN are dropped here from the keys (d_set_keys: table index |
+// empty class << 31) of the two SNPs.
+__device__ __forceinline__ bool set_pair_live(uint32_t ki, uint32_t kj) {
+    const bool rev = (ki & 0x7fffffffu) > (kj & 0x7fffffffu);
+    return ((rev ? ki : kj) >> 31) == 0;
 }
 
 // Tiles before band b. Every band before the last is full (BD A-blocks, at least BD columns): BD (TB - BD b') - BD (BD - 1) / 2 tiles.
@@ -315,6 +337,9 @@ __device__ __forceinline__ void unpack_record(const uint4 &r0, const uint4 &r1, 
 }
 
 // ---- the kernel -------------------------------------------------------------------------------------
+// SETS: set screen on a gathered sub-table -- the leader draws list positions instead of schedule indices and reads (I2, J)
+// from p.set_tiles, and a pair counts only when set_pair_wanted and set_pair_live. The whole-table instantiation is unchanged.
+template <bool SETS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MMA_THREADS, 1)
 pair_screen_mma_kernel(const __grid_constant__ CUtensorMap map_ab, const MmaParams p) {
     extern __shared__ unsigned char smem_raw[];
@@ -376,10 +401,13 @@ pair_screen_mma_kernel(const __grid_constant__ CUtensorMap map_ab, const MmaPara
                     const int slot = (int)(n_sched % SCHED_SLOTS);
                     mbar_wait_wd(&sempty[slot], ((n_sched / SCHED_SLOTS) & 1u) ^ 1u);
                     if (t >= last) { sched_publish(sched, sfull, slot, SCHED_END, 0); break; }
-                    if (!located) { cur.locate(t, p.TB, p.n_bands, p.band); located = true; }
-                    else cur.advance(t - t_cur, p.TB, p.n_bands);
-                    t_cur = t;
-                    cur.decode(p.TB, I2, J);
+                    if constexpr (SETS) { const uint2 e = p.set_tiles[t]; I2 = e.x; J = e.y; }
+                    else {
+                        if (!located) { cur.locate(t, p.TB, p.n_bands, p.band); located = true; }
+                        else cur.advance(t - t_cur, p.TB, p.n_bands);
+                        t_cur = t;
+                        cur.decode(p.TB, I2, J);
+                    }
                     sched_publish(sched, sfull, slot, I2, J);
                     ++n_sched;
                     t_next = draw();                   // in flight while this tile's loads are issued
@@ -456,6 +484,7 @@ pair_screen_mma_kernel(const __grid_constant__ CUtensorMap map_ab, const MmaPara
             // genotype labels aa <-> bb exchanged, which the statistic does not depend on, so their record is
             // loaded with the two swapped instead of re-ordering four counts per pair.
             MmaRowF A;
+            uint32_t keyA = 0;                        // SETS: this A-SNP's d_set_keys entry, carried in the record's padding
             {
                 const uint4 *rq = reinterpret_cast<const uint4 *>(p.rowf + gi);
                 const uint4 r0 = __ldg(rq), r1 = __ldg(rq + 1), r2 = __ldg(rq + 2), r3 = __ldg(rq + 3);
@@ -463,13 +492,15 @@ pair_screen_mma_kernel(const __grid_constant__ CUtensorMap map_ab, const MmaPara
                 A.pca1 = make_float2(__uint_as_float(r1.x), __uint_as_float(r1.y)); A.RA = make_float2(__uint_as_float(r1.z), __uint_as_float(r1.w));
                 A.cm0 = make_float2(__uint_as_float(r2.x), __uint_as_float(r2.y)); A.cm2 = make_float2(__uint_as_float(r2.z), __uint_as_float(r2.w));
                 A.C = __uint_as_float(r3.x);
+                if constexpr (SETS) keyA = r3.y;
                 if (pl) { float2 x = A.dA0; A.dA0 = A.dA2; A.dA2 = x; x = A.cm0; A.cm0 = A.cm2; A.cm2 = x; }
             }
             const float thr_now = sink_threshold(p.sink);
             const float thrA = thr_now / 1.3862943611f + p.q0 + A.C;   // bound pass, log2 units: N log2 tau + qc Q > thr / (2 ln 2) + q0 + C_row + C_col
             // interior tile: every pair is i < j inside the table and no block has missing calls
-            const bool interior = (uint64_t)(I + 1) * MMA_A_SNPS <= (uint64_t)J * MMA_B_SNPS && (uint64_t)(J + 1) * MMA_B_SNPS <= p.M &&
-                                  !p.tile_missing[I] && !p.tile_missing[2 * J] && !p.tile_missing[2 * J + 1];
+            bool interior = (uint64_t)(I + 1) * MMA_A_SNPS <= (uint64_t)J * MMA_B_SNPS && (uint64_t)(J + 1) * MMA_B_SNPS <= p.M &&
+                            !p.tile_missing[I] && !p.tile_missing[2 * J] && !p.tile_missing[2 * J + 1];
+            if constexpr (SETS) interior = false;     // every pair takes the set rule and set_pair_live
             const bool a_ok = (uint64_t)I * MMA_A_SNPS < p.M && !p.tile_missing[I];
             // missing-call flags of the two 64-SNP halves of the B-block (a half beyond the table counts as flagged)
             const bool b_bad0 = (uint64_t)(2 * J) * TILE >= p.M || p.tile_missing[2 * J];
@@ -524,6 +555,7 @@ pair_screen_mma_kernel(const __grid_constant__ CUtensorMap map_ab, const MmaPara
                     v[4 * s + 0] = keep0; v[4 * s + 1] = keep1; v[4 * s + 2] = got0; v[4 * s + 3] = got1;   // own plane of A first
                     const uint64_t gj = gj0 + 2 * s;
                     float2 b[7]; float Ccol;
+                    uint32_t keyB = 0;
                     {
                         const uint4 *cq = reinterpret_cast<const uint4 *>(my_col + (16 * h + 2 * s + pl) * 64);
                         const uint4 r0 = cq[0], r1 = cq[1], r2 = cq[2], r3 = cq[3];
@@ -531,9 +563,11 @@ pair_screen_mma_kernel(const __grid_constant__ CUtensorMap map_ab, const MmaPara
                         b[2] = make_float2(__uint_as_float(r1.x), __uint_as_float(r1.y)); b[3] = make_float2(__uint_as_float(r1.z), __uint_as_float(r1.w));
                         b[4] = make_float2(__uint_as_float(r2.x), __uint_as_float(r2.y)); b[5] = make_float2(__uint_as_float(r2.z), __uint_as_float(r2.w));
                         b[6] = make_float2(__uint_as_float(r3.x), __uint_as_float(r3.y)); Ccol = __uint_as_float(r3.z);
+                        if constexpr (SETS) keyB = r3.w;
                     }
                     const float ub = ksa_bound_fast(decode2(keep0), decode2(keep1), decode2(got0), decode2(got1), A, b, p.N, p.qc);
-                    const bool valid = interior | ((gi < gj) & (gj < p.M) & edge_ok);      // no short-circuit: keeps the pass branch-free
+                    const bool valid = interior | ((gi < gj) & (gj < p.M) & edge_ok &
+                                                   (!SETS || (set_pair_wanted(gi, gj, p.set_c1, p.set_a1) & set_pair_live(keyA, keyB))));   // no short-circuit: keeps the pass branch-free
                     hot |= (valid & (ub > thrA + Ccol)) ? (1u << s) : 0u;
                 }
                 // pass 2, rare: exact fp32 formula for the pairs whose bound passed
@@ -783,6 +817,9 @@ struct Mma4Params {
     float N, lnN;
     CandSink sink;
     unsigned long long *tile_counter;   // zero at launch (tile feed)
+    const uint2 *set_tiles;             // set screens (SETS instantiations; appended, as in MmaParams): the shard's tiles, n_tiles of them,
+    uint64_t set_c1, set_a1;            // the segment bounds and the sub-table's d_set_keys
+    const uint32_t *set_keys;
 };
 
 __device__ __forceinline__ uint32_t sel4(uint32_t k, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
@@ -800,7 +837,8 @@ __device__ __forceinline__ uint32_t sel4(uint32_t k, uint32_t a, uint32_t b, uin
 //                K range of a row is class-pure: the MMAs of the case sample blocks go to one, those of the control blocks
 //                to the other). Any class sizes with missing calls; the price is the accumulator double buffering (the
 //                epilogue of a tile no longer overlaps the MMAs of the next). All tiles of such a cohort take it.
-template <int MODE>
+// SETS: set screen as in pair_screen_mma_kernel; the leader walks the list and `wanted` still picks the tiles of this launch.
+template <int MODE, bool SETS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MMA_THREADS, 1)
 pair_screen_mma4_kernel(const __grid_constant__ CUtensorMap map_ab, const __grid_constant__ CUtensorMap map_b3, const Mma4Params p) {
     constexpr bool SPLIT = MODE == 1, TWOACC = MODE == 2;
@@ -854,13 +892,23 @@ pair_screen_mma4_kernel(const __grid_constant__ CUtensorMap map_ab, const __grid
             for (;;) {
                 uint32_t I2, J;
                 if (rank == 0) {
-                    const bool more = draw.next(I2, J, wanted);
+                    bool more;
+                    if constexpr (SETS) {
+                        for (;;) {
+                            const uint64_t u = atomicAdd(p.tile_counter, 1ull);
+                            more = u < p.n_tiles;
+                            if (!more) break;
+                            const uint2 e = p.set_tiles[u];
+                            I2 = e.x; J = e.y;
+                            if (wanted(I2, J)) break;
+                        }
+                    } else more = draw.next(I2, J, wanted);
                     const int slot = (int)(n_sched % SCHED_SLOTS);
                     mbar_wait_wd(&sempty[slot], ((n_sched / SCHED_SLOTS) & 1u) ^ 1u);
                     sched_publish(sched, sfull, slot, more ? I2 : SCHED_END, J);
                     if (!more) break;
                     ++n_sched;
-                    draw.prefetch();
+                    if constexpr (!SETS) draw.prefetch();
                 } else if (!sched_next(sched, sfull, sempty, n_sched, I2, J)) break;
                 const int a_row = (int)((2 * I2 + rank) * (2 * MMA_A_SNPS)), b_row = (int)(J * MMA_N + rank * MMA_B_SNPS);
                 for (uint32_t kb = 0; kb < p.NKB; kb += KPS, ++it) {
@@ -997,7 +1045,7 @@ pair_screen_mma4_kernel(const __grid_constant__ CUtensorMap map_ab, const __grid
                     for (int e = 0; e < 2; ++e) {
                         const int b_loc = 16 * g + 8 * h + 4 * e + (int)pl;
                         const uint64_t gj = (uint64_t)J * M4_BLK + b_loc;
-                        if (!(gi < gj && gj < p.M)) continue;
+                        if (!(gi < gj && gj < p.M && (!SETS || (set_pair_wanted(gi, gj, p.set_c1, p.set_a1) && set_pair_live(__ldg(p.set_keys + gi), __ldg(p.set_keys + gj)))))) continue;
                         uint32_t prod[CPB][CPB], none[3][3];                 // plane P of A is what arrived in rotation (P - o) & 3
 #pragma unroll
                         for (int P = 0; P < 4; ++P) {
@@ -1043,7 +1091,7 @@ pair_screen_mma4_kernel(const __grid_constant__ CUtensorMap map_ab, const __grid
                         }
                         const int b_loc = 16 * g + 8 * h + 4 * e + (int)pl;
                         const uint64_t gj = (uint64_t)J * M4_BLK + b_loc;
-                        if (gi < gj && gj < p.M)
+                        if (gi < gj && gj < p.M && (!SETS || (set_pair_wanted(gi, gj, p.set_c1, p.set_a1) && set_pair_live(__ldg(p.set_keys + gi), __ldg(p.set_keys + gj)))))
                             finish_pair(gj, *reinterpret_cast<const PairSide *>(my_col + (8 * h + 4 * e + (int)pl) * 128), prod, prod_ctl);
                     }
                 }
@@ -1096,8 +1144,12 @@ __global__ void expand_mma4_kernel(const uint32_t *__restrict__ sel, uint32_t se
     }
 }
 
+// SETS: records of a set screen's sub-table (set_pair_live): an empty class gives w = 0 instead of NaN, and the paddings of the
+// bound-pass records carry the SNP's d_set_keys entry (keys)
+template <bool SETS>
 __global__ void mma_side_kernel(const gwasdev_marginal_information *__restrict__ mi, uint64_t M, uint64_t Mrec, uint32_t n_ind,
-                                const uint8_t *__restrict__ derived, MmaRow *__restrict__ row, MmaCol *__restrict__ col, MmaRowF *__restrict__ rowf, MmaColF *__restrict__ colf) {
+                                const uint8_t *__restrict__ derived, MmaRow *__restrict__ row, MmaCol *__restrict__ col, MmaRowF *__restrict__ rowf, MmaColF *__restrict__ colf,
+                                const uint32_t *__restrict__ keys) {
     const uint64_t snp = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (snp >= Mrec) return;
     MmaRow r; MmaCol c;
@@ -1117,7 +1169,7 @@ __global__ void mma_side_kernel(const gwasdev_marginal_information *__restrict__
                 const int g = perm[role];
                 const double pca = m.dPca[4 * k + g], pbc = m.dPbc[4 * k + g], mar = (double)m.margins[g];
                 rp[k][role] = (float)pca;
-                cw[k][role] = m.margins[g] > 0 ? (float)(pbc / mar) : qnan;
+                cw[k][role] = m.margins[g] > 0 ? (float)(pbc / mar) : (SETS ? 0.f : qnan);
                 cn[k][role] = (float)cnt[g];
                 if (cnt[g] > 0) { Cr += (double)cnt[g] * log2(pca); Cc += (double)cnt[g] * (log2(pbc) - log2(mar)); }
             }
@@ -1163,6 +1215,10 @@ __global__ void mma_side_kernel(const gwasdev_marginal_information *__restrict__
     cf.dB0 = make_float2(db0[0], db0[1]); cf.dB2 = make_float2(db2[0], db2[1]);
     cf.w1 = make_float2(cw[0][1], cw[1][1]); cf.RB = make_float2(rb[0], rb[1]);
     cf.cm0 = make_float2(cn[0][0], (float)mp[0]); cf.cm1 = make_float2(cn[0][1], (float)mp[1]); cf.cm2 = make_float2(cn[0][2], (float)mp[2]);
+    if constexpr (SETS) {
+        const uint32_t key = snp < M ? keys[snp] : 0u;
+        rf.pad[0] = cf.pad = __uint_as_float(key);
+    }
     rowf[snp] = rf; colf[snp] = cf;
 }
 
@@ -1278,8 +1334,12 @@ static int ensure_mma_inputs(gwasdev_store *s) {
         GW_CUDA(reserve_raw(row, s->cap_mma_row, Msnp * (sizeof(MmaRow) + sizeof(MmaRowF))));
         GW_CUDA(reserve_raw(col, s->cap_mma_col, Msnp * (sizeof(MmaCol) + sizeof(MmaColF))));
         s->d_mma_row = row; s->d_mma_col = col;
-        mma_side_kernel<<<(unsigned)((Msnp + 127) / 128), 128, 0, s->stream>>>(s->d_mi, s->M, Msnp, s->n_case + s->n_ctrl, s->d_plane_derived, row, col,
-                                                                             (MmaRowF *)(row + Msnp), (MmaColF *)(col + Msnp));
+        if (s->d_set_keys)
+            mma_side_kernel<true><<<(unsigned)((Msnp + 127) / 128), 128, 0, s->stream>>>(s->d_mi, s->M, Msnp, s->n_case + s->n_ctrl, s->d_plane_derived, row, col,
+                                                                                       (MmaRowF *)(row + Msnp), (MmaColF *)(col + Msnp), s->d_set_keys);
+        else
+            mma_side_kernel<false><<<(unsigned)((Msnp + 127) / 128), 128, 0, s->stream>>>(s->d_mi, s->M, Msnp, s->n_case + s->n_ctrl, s->d_plane_derived, row, col,
+                                                                                        (MmaRowF *)(row + Msnp), (MmaColF *)(col + Msnp), nullptr);
         GW_LAUNCHED();
         s->mma_side_valid = true;
     }
@@ -1340,11 +1400,12 @@ static size_t mma_smem_bytes() {
     return 1024 + (size_t)MMA_STAGES * STAGE_BYTES_MMA + EPI_WARPS * COL_STAGE_BYTES + (2 * MMA_STAGES + 4 + 2 * SCHED_SLOTS) * sizeof(uint64_t) + SCHED_SLOTS * sizeof(uint2) + 16;
 }
 
+template <bool SETS = false>
 static int launch_mma(gwasdev_store *s, MmaParams &p, uint64_t my_tiles) {
     int sms = 0;
     GW_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
     const size_t smem = mma_smem_bytes();
-    GW_CUDA(cudaFuncSetAttribute(pair_screen_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    GW_CUDA(cudaFuncSetAttribute(pair_screen_mma_kernel<SETS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const unsigned pairs = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)sms / 2, my_tiles));   // one CTA pair per TPC
 #ifdef GWASDEV_SWEEP
     const bool prof = getenv("GWASDEV_MMA_PROF") != nullptr && !p.dump;
@@ -1360,7 +1421,7 @@ static int launch_mma(gwasdev_store *s, MmaParams &p, uint64_t my_tiles) {
     if (!s->d_tile_counter) GW_CUDA(cudaMalloc(&s->d_tile_counter, sizeof(unsigned long long)));
     GW_CUDA(cudaMemsetAsync(s->d_tile_counter, 0, sizeof(unsigned long long), s->stream));
     p.tile_counter = s->d_tile_counter;
-    pair_screen_mma_kernel<<<2 * pairs, MMA_THREADS, smem, s->stream>>>(*(const CUtensorMap *)s->tmap_mm, p);
+    pair_screen_mma_kernel<SETS><<<2 * pairs, MMA_THREADS, smem, s->stream>>>(*(const CUtensorMap *)s->tmap_mm, p);
     GW_LAUNCHED();
     if (prof) {
         std::vector<unsigned long long> h((size_t)2 * pairs * 8);
@@ -1388,6 +1449,7 @@ static void fill_params(gwasdev_store *s, MmaParams &p, uint32_t shard, uint32_t
     p.qc = s->mma_qc; p.q0 = s->mma_q0;
     p.sink = CandSink{};
     p.dump = nullptr; p.dump_tile = 0; p.dump_rank = 0; p.prof = nullptr;
+    p.set_tiles = nullptr; p.set_c1 = p.set_a1 = 0;
 }
 
 // ---- four-plane engine: host side ---------------------------------------------------------------------
@@ -1472,8 +1534,65 @@ uint64_t gwasdev_internal_mma4_shard_pairs(gwasdev_store *s, uint32_t shard, uin
     return pairs;
 }
 
+// ---- set screens: tile lists --------------------------------------------------------------------------
+// wanted pairs (set_pair_wanted) of a sub-table of M SNPs inside [i0, i1) x [j0, j1)
+static uint64_t set_rect_pairs(uint64_t M, uint64_t c1, uint64_t a1, uint64_t i0, uint64_t i1, uint64_t j0, uint64_t j1) {
+    return rect_pairs(M, i0, std::min(i1, c1), j0, j1) + rect_pairs(M, std::max(i0, c1), std::min(i1, a1), std::max(j0, a1), j1);
+}
+
+// The set screen's tiles for blocks of `blk` SNPs and bands of `band` A-blocks: the tiles of the whole-table schedule of the
+// sub-table that hold a wanted pair, in schedule order, so that the tile feed keeps its L2 banding. Shards take turns in chunks
+// of SHARD_CHUNK list positions; the shard's tiles go to `out`. Bands that start at or beyond a1 hold no wanted pair.
+static void set_tile_list(uint64_t M, uint64_t c1, uint64_t a1, uint32_t blk, uint32_t band, uint32_t shard, uint32_t n_shards,
+                          std::vector<uint2> &out) {
+    out.clear();
+    const uint32_t TB = (uint32_t)((M + blk - 1) / blk), n_bands = (TB + band - 1) / band;
+    uint64_t u = 0;
+    for (uint32_t b = 0; b < n_bands && (uint64_t)band * b * blk < a1; ++b) {
+        const uint32_t na = band_height(TB, b, band);
+        for (uint32_t J = band * b; J < TB; ++J)
+            for (uint32_t ii = 0; ii < column_height(na, J - band * b); ++ii) {
+                const uint64_t I2 = (uint64_t)band * b + ii;
+                if (set_rect_pairs(M, c1, a1, I2 * blk, (I2 + 1) * blk, (uint64_t)J * blk, (uint64_t)(J + 1) * blk) == 0) continue;
+                if (tile_in_shard(u++, shard, n_shards)) out.push_back(make_uint2((uint32_t)I2, J));
+            }
+    }
+}
+
+// The shard's tile list of the set screen for the two-plane kernel (mode -1) or the four-plane kernel in `mode` (0, 1, 2;
+// see gwasdev_internal_mma4_shard_pairs), and the wanted pairs the kernel computes in it: those of the 64-SNP blocks without
+// missing calls (two-plane; flags == nullptr: no block has any), of the tiles with (mode 0) or without (mode 1) missing calls,
+// or of every tile (mode 2). *tiles_out = tiles the kernel computes.
+uint64_t gwasdev_internal_set_shard_pairs(gwasdev_store *s, uint64_t c1, uint64_t a1, uint32_t shard, uint32_t n_shards, const uint8_t *flags,
+                                          int mode, std::vector<uint2> &list, uint64_t *tiles_out) {
+    const uint64_t M = s->M;
+    uint64_t pairs = 0, tiles = 0;
+    if (mode < 0) {
+        set_tile_list(M, c1, a1, MMA_BLK, schedule_band((uint64_t)MMA_N * 32 * s->Wr), shard, n_shards, list);
+        for (const uint2 &t : list) {
+            ++tiles;
+            for (int sa = 0; sa < 2; ++sa)
+                for (int sb = 0; sb < 2; ++sb) {
+                    const uint64_t ia = 2ull * t.x + sa, jb = 2ull * t.y + sb;
+                    if (ia * TILE < M && jb * TILE < M && (!flags || (!flags[ia] && !flags[jb])))
+                        pairs += set_rect_pairs(M, c1, a1, ia * TILE, (ia + 1) * TILE, jb * TILE, (jb + 1) * TILE);
+                }
+        }
+    } else {
+        set_tile_list(M, c1, a1, M4_BLK, m4_band(s, mode), shard, n_shards, list);
+        for (const uint2 &t : list) {
+            if (mode != 2 && ((flags[t.x] | flags[t.y]) != 0) == (mode == 1)) continue;
+            ++tiles;
+            pairs += set_rect_pairs(M, c1, a1, (uint64_t)t.x * M4_BLK, (uint64_t)(t.x + 1) * M4_BLK, (uint64_t)t.y * M4_BLK, (uint64_t)(t.y + 1) * M4_BLK);
+        }
+    }
+    if (tiles_out) *tiles_out = tiles;
+    return pairs;
+}
+
 // Launches the four-plane tensor-core screen over this shard's tiles with missing calls. thr carries the fp32 margin.
-int gwasdev_internal_screen_mma4(gwasdev_store *s, const CandSink &sink, uint32_t shard, uint32_t n_shards, int mode) {
+// set != nullptr: the set screen over the shard's list instead (shard / n_shards are then part of the list).
+int gwasdev_internal_screen_mma4(gwasdev_store *s, const CandSink &sink, uint32_t shard, uint32_t n_shards, int mode, const SetLaunch *set) {
     int rc = ensure_mma4_inputs(s, mode);
     if (rc != GWASDEV_OK) return rc;
     Mma4Params p;
@@ -1483,7 +1602,9 @@ int gwasdev_internal_screen_mma4(gwasdev_store *s, const CandSink &sink, uint32_
     const uint32_t n_ind = s->n_case + s->n_ctrl;
     p.N = (float)n_ind; p.lnN = (float)std::log((double)n_ind);
     p.sink = sink;
-    const uint64_t my_tiles = shard_tiles_before(p.n_tiles, shard, n_shards);
+    p.set_tiles = nullptr; p.set_c1 = p.set_a1 = 0; p.set_keys = s->d_set_keys;
+    if (set) { p.n_tiles = set->n_tiles; p.shard = 0; p.n_shards = 1; p.set_tiles = set->tiles; p.set_c1 = set->c1; p.set_a1 = set->a1; }
+    const uint64_t my_tiles = shard_tiles_before(p.n_tiles, p.shard, p.n_shards);
     if (my_tiles == 0) return GWASDEV_OK;
     int sms = 0;
     GW_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
@@ -1491,20 +1612,26 @@ int gwasdev_internal_screen_mma4(gwasdev_store *s, const CandSink &sink, uint32_
     if (!s->d_tile_counter) GW_CUDA(cudaMalloc(&s->d_tile_counter, sizeof(unsigned long long)));
     GW_CUDA(cudaMemsetAsync(s->d_tile_counter, 0, sizeof(unsigned long long), s->stream));
     p.tile_counter = s->d_tile_counter;
-#define SCREEN4(MODE_)                                                                                                         \
+#define SCREEN4(MODE_, SETS_)                                                                                                  \
     do {                                                                                                                       \
         const size_t smem = M4Smem<MODE_>::BYTES;                                                                              \
-        GW_CUDA(cudaFuncSetAttribute(pair_screen_mma4_kernel<MODE_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));  \
-        pair_screen_mma4_kernel<MODE_><<<2 * pairs, MMA_THREADS, smem, s->stream>>>(((const CUtensorMap *)s->tmap_mm4)[0], ((const CUtensorMap *)s->tmap_mm4)[1], p); \
+        GW_CUDA(cudaFuncSetAttribute(pair_screen_mma4_kernel<MODE_, SETS_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        pair_screen_mma4_kernel<MODE_, SETS_><<<2 * pairs, MMA_THREADS, smem, s->stream>>>(((const CUtensorMap *)s->tmap_mm4)[0], ((const CUtensorMap *)s->tmap_mm4)[1], p); \
     } while (0)
-    if (mode == 1) SCREEN4(1); else if (mode == 2) SCREEN4(2); else SCREEN4(0);
+    if (set) { if (mode == 1) SCREEN4(1, true); else if (mode == 2) SCREEN4(2, true); else SCREEN4(0, true); }
+    else if (mode == 1) SCREEN4(1, false); else if (mode == 2) SCREEN4(2, false); else SCREEN4(0, false);
 #undef SCREEN4
     GW_LAUNCHED();
     return GWASDEV_OK;
 }
 
+// operands and records of the two kernels ahead of a set screen's timed region
+int gwasdev_internal_ensure_mma(gwasdev_store *s) { return ensure_mma_inputs(s); }
+int gwasdev_internal_ensure_mma4(gwasdev_store *s, int mode) { return ensure_mma4_inputs(s, mode); }
+
 // Launches the tensor-core screen for this shard's clean tiles. thr already carries the fp32 margin.
-int gwasdev_internal_screen_mma(gwasdev_store *s, const CandSink &sink, uint32_t shard, uint32_t n_shards) {
+// set != nullptr: the set screen over the shard's list instead.
+int gwasdev_internal_screen_mma(gwasdev_store *s, const CandSink &sink, uint32_t shard, uint32_t n_shards, const SetLaunch *set) {
     const bool trace = s->opt[GWASDEV_OPT_TRACE] != 0;
     if (trace) cudaEventRecord(s->ev2, s->stream);
     int rc = ensure_mma_inputs(s);
@@ -1516,6 +1643,12 @@ int gwasdev_internal_screen_mma(gwasdev_store *s, const CandSink &sink, uint32_t
         fprintf(stderr, "[gwasdev trace] tensor-core operands + per-SNP records %.3f ms\n", ms);
     }
     MmaParams p;
+    if (set) {
+        fill_params(s, p, 0, 1);
+        p.n_tiles = set->n_tiles; p.sink = sink;
+        p.set_tiles = set->tiles; p.set_c1 = set->c1; p.set_a1 = set->a1;
+        return set->n_tiles == 0 ? GWASDEV_OK : launch_mma<true>(s, p, set->n_tiles);
+    }
     fill_params(s, p, shard, n_shards);
     const uint64_t n_tiles = s->mm_tiles;
     p.n_tiles = n_tiles;
@@ -1558,6 +1691,30 @@ int gwasdev_shard_schedule(uint64_t n_snps, uint64_t n_samples, int engine, uint
                 if (t % n_shards == shard) take(I, J, TILE);
     }
     if (n_tiles) *n_tiles = cnt;
+    if (n_pairs) *n_pairs = pairs;
+    return GWASDEV_OK;
+}
+
+int gwasdev_set_schedule(uint64_t n_snps, uint64_t n_samples, uint32_t tile_snps, const uint32_t *set_a, uint64_t n_a, const uint32_t *set_b,
+                         uint64_t n_b, uint32_t shard, uint32_t n_shards, uint32_t *tiles, uint64_t capacity, uint64_t *n_tiles, uint64_t *n_pairs) {
+    GW_REQUIRE(n_samples >= 1 && n_shards >= 1 && shard < n_shards && (tile_snps == MMA_BLK || tile_snps == M4_BLK),
+               "gwasdev_set_schedule: bad argument (tile_snps %u: 128 two-plane, 64 four-plane)", tile_snps);
+    std::vector<uint32_t> map;
+    uint64_t c1 = 0, a1 = 0;
+    int rc = gwasdev_internal_set_rows(n_snps, set_a, n_a, set_b, n_b, "gwasdev_set_schedule", map, &c1, &a1);
+    if (rc != GWASDEV_OK) return rc;
+    std::vector<uint2> list;
+    uint64_t pairs = 0;
+    if (map.size() >= 2) {
+        // the band of the screen's operand rows: one byte per raw sample position (32 * Wr, gwasdev_create's geometry)
+        const uint32_t row_bytes = 32 * round_up(plane_blocks((uint32_t)n_samples) / 2, 4);
+        set_tile_list(map.size(), c1, a1, tile_snps, schedule_band((uint64_t)MMA_N * row_bytes), shard, n_shards, list);
+        for (const uint2 &t : list)
+            pairs += set_rect_pairs(map.size(), c1, a1, (uint64_t)t.x * tile_snps, (uint64_t)(t.x + 1) * tile_snps, (uint64_t)t.y * tile_snps,
+                                    (uint64_t)(t.y + 1) * tile_snps);
+    }
+    for (uint64_t k = 0; tiles && k < std::min<uint64_t>(capacity, list.size()); ++k) { tiles[2 * k] = list[k].x; tiles[2 * k + 1] = list[k].y; }
+    if (n_tiles) *n_tiles = list.size();
     if (n_pairs) *n_pairs = pairs;
     return GWASDEV_OK;
 }

@@ -676,6 +676,21 @@ int gwasdev_select_case_control(gwasdev_store *s, const uint16_t *case_mask, con
     return GWASDEV_OK;
 }
 
+}  // extern "C"
+
+int gwasdev_internal_replay_settings(const gwasdev_store *src, gwasdev_store *dst) {
+    for (int o = 0; o < GWASDEV_OPT_COUNT; ++o) dst->opt[o] = src->opt[o];
+    dst->pair_engine = src->pair_engine;
+    dst->eager_select = src->eager_select;
+    if (src->selected && !src->h_given_masks.empty()) {
+        const uint16_t *m = src->h_given_masks.data();
+        return gwasdev_select_case_control(dst, m, m + src->P);
+    }
+    return GWASDEV_OK;
+}
+
+extern "C" {
+
 // Masks of the mask-on-the-fly overloads only (getCaseControlGenotypeDistribution(r, ccs, ..) :609-657,
 // getCaseControlContingencyTable(i, j, ccs, ..) :806-895): in the reference these never touch the pre-selected
 // m_cases_controls, so the selection, the compacted rows, the margins and the pairwise layouts all stay valid.
