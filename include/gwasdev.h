@@ -134,7 +134,16 @@ GWASDEV_API int gwasdev_pack_row_text(const char *txt, size_t len, uint32_t n_sa
  * first block), so that genotype labels stay first-seen over the whole row as in the reference. */
 GWASDEV_API int gwasdev_pack_row_text_block(const char *txt, size_t len, uint32_t n_samples, uint16_t *row,
                                 uint16_t *label_state);
-/* Upload / download n_rows rows in that layout (row stride 2P+1 blocks, host memory). */
+/* Upload / download n_rows rows in that layout (row stride 2P+1 blocks, host memory).
+ * Every call that writes rows (gwasdev_put_rows, gwasdev_put_bed, gwasdev_load_bed, gwasdev_put_tped_text, gwasdev_load_tped,
+ * gwasdev_simulate, gwasdev_simulate_block), even of a single row, drops the case/control selection and everything derived from
+ * the rows: the compacted rows, margins, pair-screen operands, cached row totals, the permutation test's SNP planes and the LD
+ * operand. Until the next gwasdev_select_case_control, every call that works on a selection fails with GWASDEV_EINVAL and returns
+ * nothing for the old one: the marginal scans (gwasdev_marginal_scan, _compact, _accumulate), gwasdev_marginal_permute,
+ * gwasdev_counts mode 2, gwasdev_pair_tables and gwasdev_epi_pairs modes 2 and 3, gwasdev_ksa, gwasdev_ksa_screen_f32,
+ * gwasdev_ksa_screen_mma_f32, gwasdev_gtest, gwasdev_mma_tile_counts, the pair screens, gwasdev_get_selected_rows and
+ * gwasdev_case_control_counts (gwasdev_is_compacted returns -1). The stream masks are over samples, not rows, and stay: modes 0 and
+ * 1 of gwasdev_counts, gwasdev_pair_tables and gwasdev_epi_pairs, gwasdev_ld_window and gwasdev_ld_pairs read the new rows. */
 GWASDEV_API int gwasdev_put_rows(gwasdev_store *s, uint64_t first_row, uint64_t n_rows, const uint16_t *rows);
 GWASDEV_API int gwasdev_get_rows(gwasdev_store *s, uint64_t first_row, uint64_t n_rows, uint16_t *rows);
 /* GenoTable::operator()(r, c) + decodeGenotype (compressed_genotype_table5.cpp:400-432,1225-1231). */
@@ -408,7 +417,9 @@ GWASDEV_API int gwasdev_set_schedule(uint64_t n_snps, uint64_t n_samples, uint32
 
 /* ---- several devices, one host process (the multi-GPU driver a C++ caller reaches) -------------------------------------
  * Copy of a store on another device: headers and raw rows travel device to device (NVLink when peer access is available),
- * options, engine choice and the current selection are re-applied. What a caller does after loading the genotype file once. */
+ * options, engine choice, selection mode, the current selection and then the current stream masks (gwasdev_set_stream_masks, which
+ * outlive a row write) are re-applied, so every call gives on the copy what it gives on src. Derived state is not copied: the copy
+ * builds it again on first use. device may be src's own device. What a caller does after loading the genotype file once. */
 GWASDEV_API int gwasdev_replicate(gwasdev_store *src, int device, gwasdev_store **out);
 /* computeBoost's pre-screen (algorithms/epistasis_func.cpp:397-486) over n_stores stores that hold the same table and
  * selection on n_stores different devices: store d runs shard d of n_stores of the tile-pair schedule on its own host thread

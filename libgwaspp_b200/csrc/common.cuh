@@ -145,6 +145,7 @@ struct gwasdev_store {
     uint32_t n_fly_case = 0, n_fly_ctrl = 0;                           // members of the on-the-fly masks as given (reference: ccs.getCaseCount() / getControlCount())
     std::vector<uint32_t> h_sel_masks;                                 // host copy of the selection masks [2][Wr]: K0's tables are built from it on demand
     std::vector<uint16_t> h_given_masks;                               // the selection's stream masks as given [2][P] (gwasdev_replicate re-applies them)
+    std::vector<uint16_t> h_fly_masks;                                 // the on-the-fly masks as given [2][P]: the selection's or gwasdev_set_stream_masks'
     // per-SNP totals over ALL samples (|p1|, |p2|, |p1 & p2|, 0), independent of the phenotype: when the classes partition the
     // cohort the control counts are totals - case counts, so a re-selection's scan needs three masked popcount streams only
     uint4 *d_row_tot = nullptr;

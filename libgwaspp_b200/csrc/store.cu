@@ -665,6 +665,7 @@ int gwasdev_select_case_control(gwasdev_store *s, const uint16_t *case_mask, con
     s->h_sel_masks.assign(mca_sel, mca_sel + 2ull * Wr);
     s->h_given_masks.assign(case_mask, case_mask + s->P);
     s->h_given_masks.insert(s->h_given_masks.end(), ctrl_mask, ctrl_mask + s->P);
+    s->h_fly_masks = s->h_given_masks;
     s->selected = true;
     s->fly_valid = true;
     s->sel_built = false;
@@ -684,7 +685,14 @@ int gwasdev_internal_replay_settings(const gwasdev_store *src, gwasdev_store *ds
     dst->eager_select = src->eager_select;
     if (src->selected && !src->h_given_masks.empty()) {
         const uint16_t *m = src->h_given_masks.data();
-        return gwasdev_select_case_control(dst, m, m + src->P);
+        const int rc = gwasdev_select_case_control(dst, m, m + src->P);
+        if (rc != GWASDEV_OK) return rc;
+    }
+    // the stream masks after the selection, which resets them: gwasdev_set_stream_masks may have replaced them since, and they
+    // outlive a row write that drops the selection
+    if (src->fly_valid && (!src->selected || src->h_fly_masks != src->h_given_masks)) {
+        const uint16_t *m = src->h_fly_masks.data();
+        return gwasdev_set_stream_masks(dst, m, m + src->P);
     }
     return GWASDEV_OK;
 }
@@ -705,6 +713,8 @@ int gwasdev_set_stream_masks(gwasdev_store *s, const uint16_t *case_mask, const 
     s->n_fly_ctrl = count_bits(m.data() + Wr, Wr);
     GW_CUDA(cudaMemcpyAsync(s->d_masks, m.data(), 2ull * Wr * sizeof(uint32_t), cudaMemcpyHostToDevice, s->stream));
     GW_CUDA(cudaStreamSynchronize(s->stream));
+    s->h_fly_masks.assign(case_mask, case_mask + s->P);
+    s->h_fly_masks.insert(s->h_fly_masks.end(), ctrl_mask, ctrl_mask + s->P);
     s->fly_valid = true;
     return GWASDEV_OK;
 }

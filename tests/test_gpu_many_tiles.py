@@ -20,8 +20,8 @@ import numpy as np
 import pytest
 
 import libgwaspp_b200 as gw
-from helpers import planted_cohort
-from test_gpu_ld import assert_band_equal, assert_records_equal, bits_of, ld_reference, ld_table, to_bed
+from helpers import bits_of, ld_reference, planted_cohort
+from test_gpu_ld import assert_band_equal, assert_records_equal, ld_table, to_bed
 from test_gpu_pair_sets import formula, in_sets
 from test_gpu_permutation import check_reductions, make_store, perm_df, pheno_of
 from test_gpu_screen_edges import LOW, store_of, top_k_of
