@@ -30,21 +30,16 @@ namespace gwasdev {
 
 constexpr int LD_A = 256;        // A-SNPs per tile: 128 per CTA (one operand row group)
 constexpr int LD_GRP = 128;      // operand row group: three rows per SNP are stored [x 128][c 128][q 128] per group of 128 SNPs
-constexpr uint32_t LD_ACC = 256; // TMEM columns per accumulator buffer
 
 template <int RT> struct LdCfg {                     // RT: operand rows per SNP (1 or 3)
     static constexpr int NB = RT == 1 ? 256 : 32;    // B-SNPs per tile
     static constexpr int KPS_ = RT == 1 ? 2 : 1;     // 128-byte sample blocks per stage
     static constexpr int STAGES = RT == 1 ? 3 : 4;
     static constexpr int A_BYTES = LD_GRP * RT * MMA_KB;     // per CTA and sample block
-    static constexpr int B_BYTES = NB / 2 * RT * MMA_KB;     // this CTA's half of B
-    static constexpr int KBB = A_BYTES + B_BYTES;
-    static constexpr int STG = KPS_ * KBB;
-    static constexpr size_t BYTES = 1024 + (size_t)STAGES * STG + (2 * STAGES + 4 + 2 * SCHED_SLOTS) * sizeof(uint64_t) +
-                                    SCHED_SLOTS * sizeof(uint2) + 16;
-    static_assert(KBB % 1024 == 0 && BYTES <= 232448, "stage blocks keep the 1 KiB swizzle alignment; at most 227 KiB per CTA");
-    static_assert(6 * NB <= (int)LD_ACC || RT == 1, "six accumulator ranges per buffer");
+    static constexpr int KBB = A_BYTES + NB / 2 * RT * MMA_KB;   // A rows, then this CTA's half of B
+    static_assert(6 * NB <= ACC_COLS || RT == 1, "six accumulator ranges per buffer");
 };
+template <int RT> using LdPipe = CtaPipe<LdCfg<RT>::STAGES, LdCfg<RT>::KPS_, LdCfg<RT>::KBB>;
 
 struct LdParams {
     uint32_t NKB;                  // 128-byte sample blocks per row
@@ -73,12 +68,6 @@ __device__ __forceinline__ void ld_stat(uint32_t n, uint32_t sx, uint32_t sy, ui
     const double dn = __ll2double_rn(num), v = __dmul_rn(__ll2double_rn(vx), __ll2double_rn(vy));
     r2 = __ddiv_rn(__dmul_rn(dn, dn), v);
     r = __ddiv_rn(dn, __dsqrt_rn(v));
-}
-
-__device__ __forceinline__ void tc_ld8(uint32_t taddr, uint32_t *v) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-                 : "r"(taddr) : "memory");
 }
 
 // one band pair of the epilogue: band entry, and a list record when r2 >= r2_min (one atomic per warp)
@@ -111,129 +100,63 @@ ld_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     using S = LdCfg<RT>;
     constexpr int NB = S::NB;
     extern __shared__ unsigned char smem_raw[];
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    unsigned char *sm = smem_raw + (base - smem_u32(smem_raw));
-    uint64_t *full = reinterpret_cast<uint64_t *>(sm + S::STAGES * S::STG);
-    uint64_t *empty = full + S::STAGES;
-    uint64_t *tfull = empty + S::STAGES;
-    uint64_t *tempty = tfull + 2;
-    uint64_t *sfull = tempty + 2;
-    uint64_t *sempty = sfull + SCHED_SLOTS;
-    uint2 *sched = reinterpret_cast<uint2 *>(sempty + SCHED_SLOTS);
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(sched + SCHED_SLOTS);
-
+    LdPipe<RT> pipe;
+    pipe.setup(smem_raw);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint32_t rank = cluster_ctarank();
-
-    if (tid == 0) {
-        for (int s = 0; s < S::STAGES; ++s) { mbar_init(&full[s], 2); mbar_init(&empty[s], 1); }
-        for (int b = 0; b < 2; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 2 * EPI_WARPS); }
-        for (int b = 0; b < SCHED_SLOTS; ++b) { mbar_init(&sfull[b], 1); mbar_init(&sempty[b], SCHED_CONSUMERS); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == MMA_WARP) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    cluster_sync_all();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t rank = pipe.rank;
+    const uint32_t tmem_base = pipe.tmem;
 
     if (warp == TMA_WARP) {
-        if (lane == 0) {
-            uint64_t it = 0;
-            uint32_t n_sched = 0;
+        // A-block-major band order; tiles past the operand's last B-block are skipped
+        auto draw = [&](uint32_t &I, uint32_t &J) -> bool {
             for (;;) {
-                uint32_t I, J;
-                if (rank == 0) {
-                    // A-block-major band order; tiles past the operand's last B-block are skipped
-                    bool more;
-                    for (;;) {
-                        const unsigned long long t = atomicAdd(p.tile_counter, 1ull);
-                        more = t < p.n_tiles;
-                        if (!more) { I = J = 0; break; }
-                        I = p.I0 + (uint32_t)(t / p.nJ);
-                        J = I * (LD_A / NB) + (uint32_t)(t % p.nJ);
-                        if (J < p.nb_blocks) break;
-                    }
-                    const int slot = (int)(n_sched % SCHED_SLOTS);
-                    mbar_wait_wd(&sempty[slot], ((n_sched / SCHED_SLOTS) & 1u) ^ 1u);
-                    sched_publish(sched, sfull, slot, more ? I : SCHED_END, J);
-                    if (!more) break;
-                    ++n_sched;
-                } else if (!sched_next(sched, sfull, sempty, n_sched, I, J)) break;
-                const uint32_t ga = 2 * I + rank;                                   // this CTA's A row group
-                const uint32_t sb = J * NB + rank * (NB / 2);                      // first B-SNP of this CTA's half
-                for (uint32_t kb = 0; kb < p.NKB; kb += S::KPS_, ++it) {
-                    const int st = (int)(it % S::STAGES);
-                    const uint32_t nk = min((uint32_t)S::KPS_, p.NKB - kb);
-                    mbar_wait_wd(&empty[st], (uint32_t)(((it / S::STAGES) & 1) ^ 1));
-                    unsigned char *dst = sm + st * S::STG;
-                    if (rank == 0) mbar_expect_tx(&full[st], nk * 2 * S::KBB);
-                    else mbar_arrive_remote(&full[st], 0);
-                    for (uint32_t k2 = 0; k2 < nk; ++k2) {
-                        const int x = (int)((kb + k2) * MMA_KB);
-                        unsigned char *d = dst + k2 * S::KBB;
-                        if constexpr (RT == 1) {
-                            tma_load_2d_pair(d, &map_a, x, (int)(ga * LD_GRP), &full[st]);
-                            tma_load_2d_pair(d + S::A_BYTES, &map_b, x, (int)sb, &full[st]);
-                        } else {
-                            const uint32_t gb = sb / LD_GRP, rb = sb % LD_GRP;
+                const unsigned long long t = atomicAdd(p.tile_counter, 1ull);
+                if (t >= p.n_tiles) { I = J = 0; return false; }
+                I = p.I0 + (uint32_t)(t / p.nJ);
+                J = I * (LD_A / NB) + (uint32_t)(t % p.nJ);
+                if (J < p.nb_blocks) return true;
+            }
+        };
+        auto load = [&](uint32_t I, uint32_t J, unsigned char *d, uint32_t blk, uint64_t *full) {
+            const uint32_t ga = 2 * I + rank;                                   // this CTA's A row group
+            const uint32_t sb = J * NB + rank * (NB / 2);                      // first B-SNP of this CTA's half
+            const int x = (int)(blk * MMA_KB);
+            if constexpr (RT == 1) {
+                tma_load_2d_pair(d, &map_a, x, (int)(ga * LD_GRP), full);
+                tma_load_2d_pair(d + S::A_BYTES, &map_b, x, (int)sb, full);
+            } else {
+                const uint32_t gb = sb / LD_GRP, rb = sb % LD_GRP;
 #pragma unroll
-                            for (int t = 0; t < 3; ++t) {
-                                tma_load_2d_pair(d + t * LD_GRP * MMA_KB, &map_a, x, (int)((3 * ga + t) * LD_GRP), &full[st]);
-                                tma_load_2d_pair(d + S::A_BYTES + t * (NB / 2) * MMA_KB, &map_b, x, (int)((3 * gb + t) * LD_GRP + rb), &full[st]);
-                            }
-                        }
-                    }
+                for (int t = 0; t < 3; ++t) {
+                    tma_load_2d_pair(d + t * LD_GRP * MMA_KB, &map_a, x, (int)((3 * ga + t) * LD_GRP), full);
+                    tma_load_2d_pair(d + S::A_BYTES + t * (NB / 2) * MMA_KB, &map_b, x, (int)((3 * gb + t) * LD_GRP + rb), full);
                 }
             }
-        }
+        };
+        pipe.produce(p.NKB, draw, load);
     } else if (warp == MMA_WARP) {
-        if (lane == 0 && rank == 0) {
-            uint64_t it = 0, tile_it = 0;
-            uint32_t n_sched = 0, I, J;
-            while (sched_next(sched, sfull, sempty, n_sched, I, J)) {
-                const uint32_t buf = (uint32_t)(tile_it & 1);
-                mbar_wait_wd(&tempty[buf], (uint32_t)(((tile_it >> 1) & 1) ^ 1));
-                tc_fence_after();
-                const uint32_t d_addr = tmem_base + buf * LD_ACC;
-                for (uint32_t kb = 0; kb < p.NKB; kb += S::KPS_, ++it) {
-                    const int st = (int)(it % S::STAGES);
-                    const uint32_t nk = min((uint32_t)S::KPS_, p.NKB - kb);
-                    mbar_wait_wd(&full[st], (uint32_t)((it / S::STAGES) & 1));
-                    tc_fence_after();
-                    for (uint32_t k2 = 0; k2 < nk; ++k2) {
-                        const uint32_t a_addr = base + st * S::STG + k2 * S::KBB, b_addr = a_addr + S::A_BYTES;
+        pipe.issue(p.NKB, [&](uint32_t d_addr, uint32_t a_addr, uint32_t blk) {
+            const uint32_t b_addr = a_addr + S::A_BYTES;
 #pragma unroll
-                        for (int k = 0; k < MMA_KB / UMMA_K; ++k) {
-                            const uint32_t acc = (kb + k2) != 0 || k != 0;
-                            const uint64_t ko = (uint64_t)(k * UMMA_K >> 4);
-                            if constexpr (RT == 1) {
-                                tc_mma_i8(d_addr, umma_desc(a_addr) + ko, umma_desc(b_addr) + ko, idesc_i8(NB), acc);
-                            } else {
-                                // per CTA, B holds [x 16][c 16][q 16]: x x (x, c), c x (x, c, q), q x c
-                                tc_mma_i8(d_addr, umma_desc(a_addr) + ko, umma_desc(b_addr) + ko, idesc_i8(2 * NB), acc);
-                                tc_mma_i8(d_addr + 2 * NB, umma_desc(a_addr + LD_GRP * MMA_KB) + ko, umma_desc(b_addr) + ko, idesc_i8(3 * NB), acc);
-                                tc_mma_i8(d_addr + 5 * NB, umma_desc(a_addr + 2 * LD_GRP * MMA_KB) + ko,
-                                          umma_desc(b_addr + (NB / 2) * MMA_KB) + ko, idesc_i8(NB), acc);
-                            }
-                        }
-                    }
-                    tc_commit_mc(&empty[st], 3);
+            for (int k = 0; k < MMA_KB / UMMA_K; ++k) {
+                const uint32_t acc = blk != 0 || k != 0;
+                const uint64_t ko = (uint64_t)(k * UMMA_K >> 4);
+                if constexpr (RT == 1) {
+                    tc_mma_i8(d_addr, umma_desc(a_addr) + ko, umma_desc(b_addr) + ko, idesc_i8(NB), acc);
+                } else {
+                    // per CTA, B holds [x 16][c 16][q 16]: x x (x, c), c x (x, c, q), q x c
+                    tc_mma_i8(d_addr, umma_desc(a_addr) + ko, umma_desc(b_addr) + ko, idesc_i8(2 * NB), acc);
+                    tc_mma_i8(d_addr + 2 * NB, umma_desc(a_addr + LD_GRP * MMA_KB) + ko, umma_desc(b_addr) + ko, idesc_i8(3 * NB), acc);
+                    tc_mma_i8(d_addr + 5 * NB, umma_desc(a_addr + 2 * LD_GRP * MMA_KB) + ko,
+                              umma_desc(b_addr + (NB / 2) * MMA_KB) + ko, idesc_i8(NB), acc);
                 }
-                tc_commit_mc(&tfull[buf], 3);
-                ++tile_it;
             }
-        }
+        });
     } else {
         // ===== epilogue (both CTAs): lane quadrant q = 32 A-SNPs of this CTA's 128, column group g = a quarter of the B-SNPs =====
         const int q = warp & 3, g = warp >> 2;
-        uint64_t tile_it = 0;
-        uint32_t n_sched = 0, I, J;
-        while (sched_next_warp(sched, sfull, sempty, lane, n_sched, I, J)) {
-            const uint32_t buf = (uint32_t)(tile_it & 1);
+        uint32_t I, J;
+        for (uint32_t tile = 0; pipe.next_warp(lane, tile, I, J); ++tile) {
             const uint64_t i = p.op0 + (uint64_t)I * LD_A + rank * LD_GRP + 32 * q + lane;   // A-SNP of this lane
             const bool i_live = i >= p.lo && i < p.a_end;
             const uint64_t iw = i - lane;                                   // the warp's A-SNPs are iw .. iw + 31
@@ -241,10 +164,8 @@ ld_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             auto outside = [&](uint64_t j0, uint32_t nj) {
                 return j0 + nj - 1 <= iw || j0 > iw + 31 + p.window || j0 >= p.hi || iw >= p.a_end || iw + 31 < p.lo;
             };
-            if (lane == 0) mbar_wait_wd(&tfull[buf], (uint32_t)((tile_it >> 1) & 1));
-            __syncwarp();
-            tc_fence_after();
-            const uint32_t taddr = tmem_base + ((uint32_t)(32 * q) << 16) + buf * LD_ACC;
+            const uint32_t buf = pipe.acc_wait(lane, tile);
+            const uint32_t taddr = tmem_base + ((uint32_t)(32 * q) << 16) + buf * ACC_COLS;
             if constexpr (RT == 1) {
                 uint2 si = make_uint2(0, 0);
                 if (i_live) si = __ldg(p.sums + i);
@@ -255,11 +176,7 @@ ld_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     tc_ld8(taddr + c0, v);
                     tc_ld8(taddr + c0 + 8, v + 8);
                     tc_wait_ld();
-                    if (h == 3) {                                  // the accumulator is in registers: hand it back before the fp64 work
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) mbar_arrive_remote(&tempty[buf], 0);
-                    }
+                    if (h == 3) pipe.acc_release(lane, buf);       // the accumulator is in registers: hand it back before the fp64 work
                     const uint64_t j0 = p.op0 + (uint64_t)J * NB + c0;
                     if (outside(j0, 16)) continue;
 #pragma unroll
@@ -281,11 +198,9 @@ ld_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                 tc_ld8(taddr + 2 * NB + 48 * h + 32 + o, cq);
                 tc_ld8(taddr + 5 * NB + 16 * h + o, qc);
                 tc_wait_ld();
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) mbar_arrive_remote(&tempty[buf], 0);
+                pipe.acc_release(lane, buf);
                 const uint64_t j0 = p.op0 + (uint64_t)J * NB + 16 * h + o;
-                if (outside(j0, 8)) { ++tile_it; continue; }
+                if (outside(j0, 8)) continue;
 #pragma unroll
                 for (int b = 0; b < 8; ++b) {
                     const uint64_t j = j0 + b;
@@ -293,16 +208,10 @@ ld_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                     ld_emit(p, ok, i, j, cc[b], xc[b], cx[b], qc[b], cq[b], xy[b], lane);
                 }
             }
-            ++tile_it;
         }
     }
 
-    tc_fence_before();
-    cluster_sync_all();
-    if (warp == MMA_WARP) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-    }
+    pipe.teardown();
 }
 
 // 32 bytes lo_bit + k * hi_bit for the 32 samples of one word
@@ -483,27 +392,14 @@ static int launch_ld(gwasdev_store *s, int RT, LdParams p, uint64_t a0, uint64_t
     p.nb_blocks = (uint32_t)((std::min(op_snps, p.hi - p.op0) + NB - 1) / NB);   // B-blocks up to the last j
     p.nJ = (uint32_t)std::min<uint64_t>((LD_A - 1 + w_eff) / NB + 1, p.nb_blocks);
     p.n_tiles = nI * p.nJ;
-    int sms = 0;
-    GW_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
-    const unsigned pairs = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)sms / 2, p.n_tiles));
-    if (!s->d_tile_counter) GW_CUDA(cudaMalloc(&s->d_tile_counter, sizeof(unsigned long long)));
-    GW_CUDA(cudaMemsetAsync(s->d_tile_counter, 0, sizeof(unsigned long long), s->stream));
-    p.tile_counter = s->d_tile_counter;
     cudaEvent_t e0, e1;
     GW_CUDA(cudaEventCreate(&e0));
     evs.push_back(e0);
     GW_CUDA(cudaEventCreate(&e1));
     evs.push_back(e1);
-    GW_CUDA(cudaEventRecord(e0, s->stream));
-#define LD_GEMM(RT_)                                                                                              \
-    do {                                                                                                          \
-        const size_t smem = LdCfg<RT_>::BYTES;                                                                    \
-        GW_CUDA(cudaFuncSetAttribute(ld_gemm_kernel<RT_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        ld_gemm_kernel<RT_><<<2 * pairs, MMA_THREADS, smem, s->stream>>>(maps[0], maps[1], p);                   \
-    } while (0)
-    if (RT == 3) LD_GEMM(3); else LD_GEMM(1);
-#undef LD_GEMM
-    GW_LAUNCHED();
+    rc = RT == 3 ? launch_cta_pairs(s, ld_gemm_kernel<3>, LdPipe<3>::SMEM, p.n_tiles, p, nullptr, e0, maps[0], maps[1])
+                 : launch_cta_pairs(s, ld_gemm_kernel<1>, LdPipe<1>::SMEM, p.n_tiles, p, nullptr, e0, maps[0], maps[1]);
+    if (rc != GWASDEV_OK) return rc;
     GW_CUDA(cudaEventRecord(e1, s->stream));
     return GWASDEV_OK;
 }

@@ -1,5 +1,6 @@
-// tcgen05 building blocks shared by the tensor-core kernels (pairwise_mma.cu: the pair screens; permute.cu: the permutation
-// test): CTA-pair geometry, PTX wrappers, the mbarrier helpers, the tile feed and the UMMA descriptors.
+// tcgen05 building blocks shared by the tensor-core kernels (pairwise_mma.cu: the pair screens; permute_gemm.cuh: the
+// permutation test; ld.cu: windowed LD): CTA-pair geometry, PTX wrappers, the mbarrier helpers, the tile feed, the UMMA
+// descriptors, and the CTA-pair pipeline (CtaPipe) with its host launch.
 #pragma once
 
 #include "pair_common.cuh"
@@ -15,7 +16,6 @@ constexpr int MMA_STAGES = 3;
 constexpr int KPS = 2;                                             // 128-byte sample blocks per stage (fewer barrier round trips)
 constexpr int A_STAGE_BYTES = 2 * MMA_A_SNPS * MMA_KB, B_STAGE_BYTES = MMA_B_SNPS * MMA_KB;   // per CTA and sample block: its A rows, its half of B
 constexpr int KB_BYTES = A_STAGE_BYTES + B_STAGE_BYTES;            // 32 KiB per CTA and sample block
-constexpr int STAGE_BYTES_MMA = KPS * KB_BYTES;                    // 64 KiB per CTA
 constexpr int EPI_WARPS = 16;
 constexpr int MMA_THREADS = (2 + EPI_WARPS) * 32;
 // The warp scheduler favours the highest warp ids: the two single-thread roles that every stage waits on sit
@@ -77,6 +77,20 @@ __device__ __forceinline__ void tc_ld24(uint32_t taddr, uint32_t (&v)[32]) {
         : "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23])
         : "r"(taddr + 16u) : "memory");
 }
+// 8 / 16 accumulator columns of this warp's 32 lanes
+__device__ __forceinline__ void tc_ld8(uint32_t taddr, uint32_t *v) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
+                 : "r"(taddr) : "memory");
+}
+__device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&v)[32]) {
+    asm volatile(
+        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
+        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
+          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
+        : "r"(taddr) : "memory");
+}
 __device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&v)[32]) {
     asm volatile(
         "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
@@ -89,6 +103,14 @@ __device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&v)[32]) {
         : "r"(taddr) : "memory");
 }
 __device__ __forceinline__ void tc_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// all 512 TMEM columns of the CTA, by one whole warp in both CTAs of the pair
+__device__ __forceinline__ void tmem_alloc_pair(uint32_t *slot) {
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(512) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc_pair(uint32_t tmem) {
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512) : "memory");
+}
 
 // mbarrier wait with a watchdog: a broken pipeline traps instead of hanging the device
 __device__ __forceinline__ void mbar_wait_wd(uint64_t *bar, uint32_t parity) {
@@ -143,18 +165,17 @@ __device__ __forceinline__ void sched_publish(uint2 *slots, uint64_t *sfull, int
         "mbarrier.arrive.release.cta.shared::cta.b64 _, [%1];\n\t}"
         ::"r"(smem_u32(&slots[slot])), "r"(smem_u32(&sfull[slot])), "r"(I2), "r"(J) : "memory");
 }
-// single-thread consumer: next tile of the pair, false at the end of the shard
-__device__ __forceinline__ bool sched_next(const uint2 *slots, uint64_t *sfull, uint64_t *sempty, uint32_t &n, uint32_t &I2, uint32_t &J) {
+// single-thread consumer: tile n of the pair (the caller counts), false at the end of the shard
+__device__ __forceinline__ bool sched_next(const uint2 *slots, uint64_t *sfull, uint64_t *sempty, uint32_t n, uint32_t &I2, uint32_t &J) {
     const int slot = (int)(n % SCHED_SLOTS);
     mbar_wait_wd_cluster(&sfull[slot], (n / SCHED_SLOTS) & 1u);
     asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(I2), "=r"(J) : "r"(smem_u32(&slots[slot])) : "memory");
     if (I2 == SCHED_END) return false;
     mbar_arrive_remote(&sempty[slot], 0);
-    ++n;
     return true;
 }
-// warp-wide consumer (epilogue): lane 0 waits and releases
-__device__ __forceinline__ bool sched_next_warp(const uint2 *slots, uint64_t *sfull, uint64_t *sempty, int lane, uint32_t &n, uint32_t &I2, uint32_t &J) {
+// warp-wide consumer (epilogue): tile n of the pair (the caller counts), lane 0 waits and releases
+__device__ __forceinline__ bool sched_next_warp(const uint2 *slots, uint64_t *sfull, uint64_t *sempty, int lane, uint32_t n, uint32_t &I2, uint32_t &J) {
     const int slot = (int)(n % SCHED_SLOTS);
     if (lane == 0) mbar_wait_wd_cluster(&sfull[slot], (n / SCHED_SLOTS) & 1u);
     __syncwarp();
@@ -162,7 +183,6 @@ __device__ __forceinline__ bool sched_next_warp(const uint2 *slots, uint64_t *sf
     __syncwarp();
     if (I2 == SCHED_END) return false;
     if (lane == 0) mbar_arrive_remote(&sempty[slot], 0);
-    ++n;
     return true;
 }
 
@@ -181,8 +201,181 @@ constexpr uint32_t idesc_i8(int n) { return (2u << 4) | (1u << 7) | (1u << 10) |
 constexpr uint32_t IDESC_I8 = idesc_i8(MMA_N);
 
 // 2-D tensor map over `rows` operand rows of `kbytes` bytes (K-major, SWIZZLE_128B boxes of 128 bytes x box_rows), as the
-// permutation test and the LD kernel stage them (permute.cu)
+// tensor-core kernels stage them (pairwise.cu)
 int encode_operand_map(void *ptr, uint64_t rows, uint32_t kbytes, uint32_t box_rows, CUtensorMap *out);
+
+#ifdef GWASDEV_SWEEP
+#define GW_PROF(x) x
+#else
+#define GW_PROF(x)
+#endif
+
+// ---- the CTA-pair pipeline --------------------------------------------------------------------------
+// Every tensor-core kernel (the pair screens, the permutation GEMM, the LD GEMM) is a persistent 2-CTA cluster of 18 warps:
+//   warp 16 (TMA_WARP)  producer: both CTAs load their rows of each stage; the loads complete on the leader's full[stage]
+//   warp 17 (MMA_WARP)  issuer  : (leader only) the MMAs of a stage into the tile's TMEM accumulator; tcgen05.commit multicasts
+//                                 empty[stage] and, at the end of the tile, tfull[acc] to both CTAs
+//   warps 0-15          epilogue: wait tfull[acc], read TMEM, release tempty[acc] to the leader, then the kernel's own work
+// over the tiles that the leader's producer draws and publishes through the tile feed above. CtaPipe holds this protocol; a
+// kernel supplies only its draw, its loads of one 128-byte sample block, its MMAs of one sample block and its epilogue.
+template <int STAGES> struct PipeBars {
+    uint64_t full[STAGES];            // the leader's arrive.expect_tx + the peer producer's arrive; both CTAs' TMA bytes land on it
+    uint64_t empty[STAGES];           // one multicast tcgen05.commit
+    uint64_t tfull[2];                // one multicast tcgen05.commit
+    uint64_t tempty[2];               // every epilogue warp of both CTAs
+    uint64_t sfull[SCHED_SLOTS];      // tile feed: slot published / slot read by every consumer of the pair
+    uint64_t sempty[SCHED_SLOTS];
+    uint2 sched[SCHED_SLOTS];
+    uint32_t tmem_slot;
+};
+// dynamic shared memory of a kernel: 1 KiB alignment slack, the stage ring, the kernel's own region, the barriers
+constexpr size_t pipe_smem_bytes(int stages, int stage_bytes, int extra_bytes) {
+    return 1024 + (size_t)stages * stage_bytes + extra_bytes + (2 * stages + 4 + 2 * SCHED_SLOTS) * sizeof(uint64_t) +
+           SCHED_SLOTS * sizeof(uint2) + 16;
+}
+
+// One CTA of the pair. STAGES stages of KPS_ sample blocks of KBB bytes (this CTA's A rows, then its half of B); EXTRA bytes
+// of the kernel's own between the ring and the barriers; NACC accumulators of ACC_COLS TMEM columns in flight (1: the epilogue
+// of a tile does not overlap the MMAs of the next).
+template <int STAGES, int KPS_, int KBB, int EXTRA = 0, int NACC = 2>
+struct CtaPipe {
+    static constexpr int STG = KPS_ * KBB;
+    static constexpr size_t SMEM = pipe_smem_bytes(STAGES, STG, EXTRA);
+    static_assert(KBB % 1024 == 0 && SMEM <= 232448, "stage blocks keep the 1 KiB swizzle alignment; at most 227 KiB per CTA");
+    unsigned char *sm;                // stage ring (SWIZZLE_128B atoms are 1024-byte aligned)
+    uint32_t base;                    // its shared address
+    PipeBars<STAGES> *bar;
+    uint32_t tmem, rank;              // rank 0: leader of the pair (issues the MMAs, owns full / tempty)
+
+    // barriers, TMEM and the cluster sync of both CTAs; returns the kernel's EXTRA bytes
+    __device__ __forceinline__ unsigned char *setup(unsigned char *smem_raw) {
+        base = (smem_u32(smem_raw) + 1023u) & ~1023u;
+        sm = smem_raw + (base - smem_u32(smem_raw));
+        bar = reinterpret_cast<PipeBars<STAGES> *>(sm + STAGES * STG + EXTRA);
+        rank = cluster_ctarank();
+        if (threadIdx.x == 0) {
+            for (int s = 0; s < STAGES; ++s) { mbar_init(&bar->full[s], 2); mbar_init(&bar->empty[s], 1); }
+            for (int b = 0; b < 2; ++b) { mbar_init(&bar->tfull[b], 1); mbar_init(&bar->tempty[b], 2 * EPI_WARPS); }
+            for (int b = 0; b < SCHED_SLOTS; ++b) { mbar_init(&bar->sfull[b], 1); mbar_init(&bar->sempty[b], SCHED_CONSUMERS); }
+            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        }
+        if (threadIdx.x / 32 == MMA_WARP) tmem_alloc_pair(&bar->tmem_slot);   // both accumulators
+        tc_fence_before();
+        cluster_sync_all();                            // barriers initialised and TMEM allocated in both CTAs
+        tc_fence_after();
+        tmem = bar->tmem_slot;
+        return sm + STAGES * STG;
+    }
+    __device__ __forceinline__ void teardown() {
+        tc_fence_before();
+        cluster_sync_all();                            // neither CTA leaves while its pair may still touch its SM
+        if (threadIdx.x / 32 == MMA_WARP) { tc_fence_after(); tmem_dealloc_pair(tmem); }
+    }
+
+    // Producer (lane 0 of TMA_WARP in both CTAs). The leader takes its tiles from draw(I, J) -> false at the end and publishes
+    // them; the peer reads them from the feed. load(I, J, dst, blk, full) issues this CTA's loads of sample block blk into dst.
+    // prof (role timers, GWASDEV_SWEEP builds): per CTA, [5] = clocks spent waiting for empty.
+    template <class Draw, class Load>
+    __device__ __forceinline__ void produce(uint32_t NKB, Draw &&draw, Load &&load, unsigned long long *prof = nullptr) {
+        if (threadIdx.x % 32 != 0) return;
+        uint64_t it = 0;
+        GW_PROF(long long prof_pw = 0;)
+        for (uint32_t tile = 0;; ++tile) {
+            uint32_t I = 0, J = 0;
+            if (rank == 0) {
+                const bool more = draw(I, J);
+                const int slot = (int)(tile % SCHED_SLOTS);
+                mbar_wait_wd(&bar->sempty[slot], ((tile / SCHED_SLOTS) & 1u) ^ 1u);
+                sched_publish(bar->sched, bar->sfull, slot, more ? I : SCHED_END, J);
+                if (!more) break;
+            } else if (!sched_next(bar->sched, bar->sfull, bar->sempty, tile, I, J)) break;
+            for (uint32_t kb = 0; kb < NKB; kb += KPS_, ++it) {
+                const int st = (int)(it % STAGES);
+                const uint32_t nk = min((uint32_t)KPS_, NKB - kb);
+                GW_PROF(const long long w0 = clock64();)
+                mbar_wait_wd(&bar->empty[st], (uint32_t)(((it / STAGES) & 1) ^ 1));
+                GW_PROF(prof_pw += clock64() - w0;)
+                if (rank == 0) mbar_expect_tx(&bar->full[st], nk * 2 * KBB);
+                else mbar_arrive_remote(&bar->full[st], 0);
+                for (uint32_t k2 = 0; k2 < nk; ++k2) load(I, J, sm + st * STG + k2 * KBB, kb + k2, &bar->full[st]);
+            }
+        }
+        GW_PROF(if (prof) prof[blockIdx.x * 8 + 5] = (unsigned long long)prof_pw;)
+        (void)prof;
+    }
+
+    // MMA issuer (lane 0 of MMA_WARP in the leader). mma(d, a, blk) issues the MMAs of sample block blk of the tile, whose
+    // stage block starts at shared address a, into the accumulator at TMEM address d (accumulating unless blk is the first).
+    // prof: [0] busy, [1] waiting for tempty, [2] waiting for full, [6] tiles.
+    template <class Mma>
+    __device__ __forceinline__ void issue(uint32_t NKB, Mma &&mma, unsigned long long *prof = nullptr) {
+        if (threadIdx.x % 32 != 0 || rank != 0) return;
+        uint64_t it = 0;
+        uint32_t tile = 0, I, J;
+        GW_PROF(long long prof_te = 0; long long prof_fu = 0; const long long prof_t0 = clock64();)
+        for (; sched_next(bar->sched, bar->sfull, bar->sempty, tile, I, J); ++tile) {
+            const uint32_t buf = tile % NACC;
+            GW_PROF(const long long w0 = clock64();)
+            mbar_wait_wd(&bar->tempty[buf], ((tile / NACC) & 1u) ^ 1u);
+            GW_PROF(prof_te += clock64() - w0;)
+            tc_fence_after();
+            const uint32_t d_addr = tmem + buf * ACC_COLS;
+            for (uint32_t kb = 0; kb < NKB; kb += KPS_, ++it) {
+                const int st = (int)(it % STAGES);
+                const uint32_t nk = min((uint32_t)KPS_, NKB - kb);
+                GW_PROF(const long long w1 = clock64();)
+                mbar_wait_wd(&bar->full[st], (uint32_t)((it / STAGES) & 1));
+                GW_PROF(prof_fu += clock64() - w1;)
+                tc_fence_after();
+                for (uint32_t k2 = 0; k2 < nk; ++k2) mma(d_addr, base + st * STG + k2 * KBB, kb + k2);
+                tc_commit_mc(&bar->empty[st], 3);      // stage reusable in both CTAs once these MMAs have read it
+            }
+            tc_commit_mc(&bar->tfull[buf], 3);         // accumulator complete in both CTAs
+        }
+        GW_PROF(if (prof) {
+            unsigned long long *o = prof + blockIdx.x * 8;
+            o[0] = (unsigned long long)(clock64() - prof_t0); o[1] = (unsigned long long)prof_te; o[2] = (unsigned long long)prof_fu; o[6] = tile;
+        })
+        (void)prof;
+    }
+
+    // Epilogue warps, counting the pair's tiles n = 0, 1, ...: tile n (false at the end), wait for its accumulator (returns its
+    // index; TMEM address tmem + index * ACC_COLS), and hand the accumulator back once its TMEM loads have completed.
+    __device__ __forceinline__ bool next_warp(int lane, uint32_t n, uint32_t &I, uint32_t &J) {
+        return sched_next_warp(bar->sched, bar->sfull, bar->sempty, lane, n, I, J);
+    }
+    __device__ __forceinline__ uint32_t acc_wait(int lane, uint64_t n) {
+        const uint32_t buf = (uint32_t)(n % NACC);
+        if (lane == 0) mbar_wait_wd(&bar->tfull[buf], (uint32_t)((n / NACC) & 1));
+        __syncwarp();
+        tc_fence_after();
+        return buf;
+    }
+    __device__ __forceinline__ void acc_release(int lane, uint32_t buf) {
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive_remote(&bar->tempty[buf], 0);
+    }
+};
+
+// Launches a CtaPipe kernel on one CTA pair per TPC, at most one pair per tile, with p.tile_counter zeroed; *pairs_out = the
+// pairs. `start` (or nullptr) is recorded right before the kernel, so that an event pair around it times the kernel alone.
+template <class Kernel, class Params, class... Maps>
+int launch_cta_pairs(gwasdev_store *s, Kernel kernel, size_t smem, uint64_t n_tiles, Params &p, unsigned *pairs_out, cudaEvent_t start,
+                     const Maps &...maps) {
+    int sms = 0;
+    GW_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
+    const unsigned pairs = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)sms / 2, n_tiles));
+    if (pairs_out) *pairs_out = pairs;
+    if (!s->d_tile_counter) GW_CUDA(cudaMalloc(&s->d_tile_counter, sizeof(unsigned long long)));
+    GW_CUDA(cudaMemsetAsync(s->d_tile_counter, 0, sizeof(unsigned long long), s->stream));
+    p.tile_counter = s->d_tile_counter;
+    GW_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (start) GW_CUDA(cudaEventRecord(start, s->stream));
+    kernel<<<2 * pairs, MMA_THREADS, smem, s->stream>>>(maps..., p);
+    GW_LAUNCHED();
+    return GWASDEV_OK;
+}
 
 __device__ __forceinline__ uint32_t spread4(uint32_t nibble) { return (nibble * 0x00204081u) & 0x01010101u; }   // bit i -> byte i
 

@@ -15,13 +15,12 @@
 //     D[2i+p][2j+q] = sum_samples A*B = n_case(p, q) + 16384 * n_ctrl(p, q)
 // exactly in int32 (n_case < 16384, n_ctrl < 131072): one accumulator tile carries both classes.
 //
-// Kernel. Two CTAs on the two SMs of a TPC work as a pair (cluster of 2, tcgen05 cta_group::2), persistent
-// over tile pairs of (128 A-SNPs = 256 rows, 128 per CTA) x (128 B-SNPs = 256 rows, each CTA stages half):
-//   warp 16  TMA producer : cp.async.bulk.tensor.2d.cta_group::2, SWIZZLE_128B boxes of 128 sample bytes, both
-//                           CTAs' loads complete on the leader's mbarrier, 6-stage ring of 32 KiB per CTA
-//   warp 17  MMA issuer   : (leader CTA) tcgen05.mma.cta_group::2.kind::i8, M=256 N=256 K=32, 4 per stage, into
-//                           one of two 256-column TMEM accumulators; tcgen05.commit multicasts "stage free" and
-//                           "accumulator ready" to both CTAs
+// Kernel. The CTA-pair pipeline of mma_common.cuh (CtaPipe), persistent over tile pairs of (128 A-SNPs = 256 rows,
+// 128 per CTA) x (128 B-SNPs = 256 rows, each CTA stages half):
+//   loads                 : 2-D SWIZZLE_128B boxes of 128 sample bytes x 128 rows, a CTA's A rows and its half of B;
+//                           three stages of two sample blocks, 64 KiB per CTA
+//   MMAs                  : tcgen05.mma.cta_group::2.kind::i8, M=256 N=256 K=32, 4 per sample block, into one of
+//                           two 256-column TMEM accumulators
 //   warps 0-15 epilogue   : each CTA reads its 128 accumulator rows (64 A-SNPs) with tcgen05.ld 32x32b, lane
 //                           pairs swap the two planes by shuffle, decode the counts, margins -> 3x3x2 table,
 //                           upper bound of the KSA statistic, exact fp32 KSA for the few that pass it,
@@ -97,12 +96,6 @@ struct MmaParams {
     const uint2 *set_tiles;
     uint64_t set_c1, set_a1;
 };
-#ifdef GWASDEV_SWEEP
-#define GW_PROF(x) x
-#else
-#define GW_PROF(x)
-#endif
-
 
 // ---- tile order -------------------------------------------------------------------------------------
 // Tiles are pairs of 128-SNP blocks (I2 <= J). Band b holds A-blocks [BD b, BD b + BD) for the band height BD of the launch;
@@ -339,133 +332,61 @@ __device__ __forceinline__ void unpack_record(const uint4 &r0, const uint4 &r1, 
 // ---- the kernel -------------------------------------------------------------------------------------
 // SETS: set screen on a gathered sub-table -- the leader draws list positions instead of schedule indices and reads (I2, J)
 // from p.set_tiles, and a pair counts only when set_pair_wanted and set_pair_live. The whole-table instantiation is unchanged.
+using MmaPipe = CtaPipe<MMA_STAGES, KPS, KB_BYTES, EPI_WARPS * COL_STAGE_BYTES>;   // extra: per epilogue warp, 32 column-role records
+
 template <bool SETS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MMA_THREADS, 1)
 pair_screen_mma_kernel(const __grid_constant__ CUtensorMap map_ab, const MmaParams p) {
     extern __shared__ unsigned char smem_raw[];
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;              // SWIZZLE_128B atoms are 1024-byte aligned
-    unsigned char *sm = smem_raw + (base - smem_u32(smem_raw));
-    unsigned char *col_sm = sm + MMA_STAGES * STAGE_BYTES_MMA;                 // per epilogue warp: 32 column-role records
-    uint64_t *full = reinterpret_cast<uint64_t *>(col_sm + EPI_WARPS * COL_STAGE_BYTES);
-    uint64_t *empty = full + MMA_STAGES;
-    uint64_t *tfull = empty + MMA_STAGES;
-    uint64_t *tempty = tfull + 2;
-    uint64_t *sfull = tempty + 2;                      // tile feed (see above): slot published / slot read by every consumer of the pair
-    uint64_t *sempty = sfull + SCHED_SLOTS;
-    uint2 *sched = reinterpret_cast<uint2 *>(sempty + SCHED_SLOTS);
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(sched + SCHED_SLOTS);
-
+    MmaPipe pipe;
+    unsigned char *col_sm = pipe.setup(smem_raw);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint32_t rank = cluster_ctarank();          // 0: leader of the CTA pair (issues the MMAs, owns full / tempty)
-
-    if (tid == 0) {
-        // full: the leader's own arrive.expect_tx + the peer producer's arrive; both CTAs' TMA bytes land on it.
-        // empty / tfull: one multicast tcgen05.commit each. tempty: every epilogue warp of both CTAs.
-        for (int s = 0; s < MMA_STAGES; ++s) { mbar_init(&full[s], 2); mbar_init(&empty[s], 1); }
-        for (int b = 0; b < 2; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 2 * EPI_WARPS); }
-        for (int b = 0; b < SCHED_SLOTS; ++b) { mbar_init(&sfull[b], 1); mbar_init(&sempty[b], SCHED_CONSUMERS); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == MMA_WARP) {   // whole warp, in both CTAs: all 512 TMEM columns (two accumulators)
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    cluster_sync_all();                                // barriers initialised and TMEM allocated in both CTAs
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t rank = pipe.rank;
+    const uint32_t tmem_base = pipe.tmem;
 
     // The shard's tiles have local indices u = 0, 1, ...; shard_tile(u) is the schedule index. Shards own alternating chunks
     // of SHARD_CHUNK consecutive tiles, so that the tiles a GPU works on at the same time share A- and B-blocks in its L2
-    // whatever the number of GPUs. The pair draws its u from p.tile_counter (tile feed above).
+    // whatever the number of GPUs. The pair draws its u from p.tile_counter (tile feed).
     const uint64_t last = p.dump ? p.dump_tile + 1 : p.n_tiles;
 
     if (warp == TMA_WARP) {
         // ===== TMA producer (both CTAs: own 128 A rows, own half of the 256 B rows) =====
-        if (lane == 0) {
-            uint64_t it = 0;
-            GW_PROF(long long prof_pw = 0;)
-            TileCursor cur;
-            uint32_t n_sched = 0, dump_u = 0;
-            uint64_t t_cur = 0;
-            bool located = false;
-            auto draw = [&]() -> uint64_t {            // schedule index of the next tile of the shard (leader only)
-                if (p.dump) return p.dump_tile + dump_u++;
-                return shard_tile(atomicAdd(p.tile_counter, 1ull), p.shard, p.n_shards);
-            };
-            uint64_t t_next = rank == 0 ? draw() : 0;
-            for (;;) {
-                uint32_t I2, J;
-                if (rank == 0) {
-                    const uint64_t t = t_next;
-                    const int slot = (int)(n_sched % SCHED_SLOTS);
-                    mbar_wait_wd(&sempty[slot], ((n_sched / SCHED_SLOTS) & 1u) ^ 1u);
-                    if (t >= last) { sched_publish(sched, sfull, slot, SCHED_END, 0); break; }
-                    if constexpr (SETS) { const uint2 e = p.set_tiles[t]; I2 = e.x; J = e.y; }
-                    else {
-                        if (!located) { cur.locate(t, p.TB, p.n_bands, p.band); located = true; }
-                        else cur.advance(t - t_cur, p.TB, p.n_bands);
-                        t_cur = t;
-                        cur.decode(p.TB, I2, J);
-                    }
-                    sched_publish(sched, sfull, slot, I2, J);
-                    ++n_sched;
-                    t_next = draw();                   // in flight while this tile's loads are issued
-                } else if (!sched_next(sched, sfull, sempty, n_sched, I2, J)) break;
-                const int a_row = (int)((2 * I2 + rank) * (2 * MMA_A_SNPS)), b_row = (int)(J * MMA_N + rank * MMA_B_SNPS);
-                for (uint32_t kb = 0; kb < p.NKB; kb += KPS, ++it) {
-                    const int st = (int)(it % MMA_STAGES);
-                    const uint32_t nk = min((uint32_t)KPS, p.NKB - kb);
-                    GW_PROF(const long long w0 = clock64();)
-                    mbar_wait_wd(&empty[st], (uint32_t)(((it / MMA_STAGES) & 1) ^ 1));
-                    GW_PROF(prof_pw += clock64() - w0;)
-                    unsigned char *dst = sm + st * STAGE_BYTES_MMA;
-                    if (rank == 0) mbar_expect_tx(&full[st], nk * 2 * KB_BYTES);
-                    else mbar_arrive_remote(&full[st], 0);
-                    for (uint32_t k2 = 0; k2 < nk; ++k2) {
-                        tma_load_2d_pair(dst + k2 * KB_BYTES, &map_ab, (int)((kb + k2) * MMA_KB), a_row, &full[st]);
-                        tma_load_2d_pair(dst + k2 * KB_BYTES + A_STAGE_BYTES, &map_ab, (int)((kb + k2) * MMA_KB), b_row, &full[st]);
-                    }
-                }
+        TileCursor cur;
+        uint32_t dump_u = 0;
+        uint64_t t_cur = 0;
+        bool located = false;
+        auto next_t = [&]() -> uint64_t {              // schedule index of the next tile of the shard (leader only)
+            if (p.dump) return p.dump_tile + dump_u++;
+            return shard_tile(atomicAdd(p.tile_counter, 1ull), p.shard, p.n_shards);
+        };
+        uint64_t t_next = rank == 0 && lane == 0 ? next_t() : 0;   // the leader's producer thread draws one tile ahead
+        auto draw = [&](uint32_t &I2, uint32_t &J) -> bool {
+            const uint64_t t = t_next;
+            if (t >= last) return false;
+            if constexpr (SETS) { const uint2 e = p.set_tiles[t]; I2 = e.x; J = e.y; }
+            else {
+                if (!located) { cur.locate(t, p.TB, p.n_bands, p.band); located = true; }
+                else cur.advance(t - t_cur, p.TB, p.n_bands);
+                t_cur = t;
+                cur.decode(p.TB, I2, J);
             }
-            GW_PROF(if (p.prof) p.prof[blockIdx.x * 8 + 5] = (unsigned long long)prof_pw;)
-        }
+            t_next = next_t();                         // in flight while this tile is published and its loads are issued
+            return true;
+        };
+        auto load = [&](uint32_t I2, uint32_t J, unsigned char *dst, uint32_t blk, uint64_t *full) {
+            const int a_row = (int)((2 * I2 + rank) * (2 * MMA_A_SNPS)), b_row = (int)(J * MMA_N + rank * MMA_B_SNPS);
+            tma_load_2d_pair(dst, &map_ab, (int)(blk * MMA_KB), a_row, full);
+            tma_load_2d_pair(dst + A_STAGE_BYTES, &map_ab, (int)(blk * MMA_KB), b_row, full);
+        };
+        pipe.produce(p.NKB, draw, load, p.prof);
     } else if (warp == MMA_WARP) {
         // ===== MMA issuer (leader CTA only) =====
-        if (lane == 0 && rank == 0) {
-            uint64_t it = 0, tile_it = 0;
-            GW_PROF(long long prof_te = 0; long long prof_fu = 0; const long long prof_t0 = clock64();)
-            uint32_t n_sched = 0, I2_, J_;
-            for (; sched_next(sched, sfull, sempty, n_sched, I2_, J_); ++tile_it) {
-                const uint32_t buf = (uint32_t)(tile_it & 1);
-                GW_PROF(const long long w0 = clock64();)
-                mbar_wait_wd(&tempty[buf], (uint32_t)(((tile_it >> 1) & 1) ^ 1));
-                GW_PROF(prof_te += clock64() - w0;)
-                tc_fence_after();
-                const uint32_t d_addr = tmem_base + buf * ACC_COLS;
-                for (uint32_t kb = 0; kb < p.NKB; kb += KPS, ++it) {
-                    const int st = (int)(it % MMA_STAGES);
-                    const uint32_t nk = min((uint32_t)KPS, p.NKB - kb);
-                    GW_PROF(const long long w1 = clock64();)
-                    mbar_wait_wd(&full[st], (uint32_t)((it / MMA_STAGES) & 1));
-                    GW_PROF(prof_fu += clock64() - w1;)
-                    tc_fence_after();
-                    for (uint32_t k2 = 0; k2 < nk; ++k2) {
-                        const uint32_t a_addr = base + st * STAGE_BYTES_MMA + k2 * KB_BYTES, b_addr = a_addr + A_STAGE_BYTES;
-                        const uint64_t ad = umma_desc(a_addr), bd = umma_desc(b_addr);
+        pipe.issue(p.NKB, [&](uint32_t d_addr, uint32_t a_addr, uint32_t blk) {
+            const uint64_t ad = umma_desc(a_addr), bd = umma_desc(a_addr + A_STAGE_BYTES);
 #pragma unroll
-                        for (int k = 0; k < MMA_KB / UMMA_K; ++k)
-                            tc_mma_i8(d_addr, ad + (uint64_t)(k * UMMA_K >> 4), bd + (uint64_t)(k * UMMA_K >> 4), IDESC_I8, (kb | k2 | (uint32_t)k) != 0);
-                    }
-                    tc_commit_mc(&empty[st], 3);      // stage reusable in both CTAs once these MMAs have read it
-                }
-                tc_commit_mc(&tfull[buf], 3);         // accumulator complete in both CTAs
-            }
-            GW_PROF(if (p.prof) {
-                unsigned long long *o = p.prof + blockIdx.x * 8;
-                o[0] = (unsigned long long)(clock64() - prof_t0); o[1] = (unsigned long long)prof_te; o[2] = (unsigned long long)prof_fu; o[6] = tile_it;
-            })
-        }
+            for (int k = 0; k < MMA_KB / UMMA_K; ++k)
+                tc_mma_i8(d_addr, ad + (uint64_t)(k * UMMA_K >> 4), bd + (uint64_t)(k * UMMA_K >> 4), IDESC_I8, (blk | (uint32_t)k) != 0);
+        }, p.prof);
     } else {
         // ===== epilogue (both CTAs: own 64 A-SNPs x the tile's 128 B-SNPs) =====
         const int ew = warp;
@@ -473,12 +394,10 @@ pair_screen_mma_kernel(const __grid_constant__ CUtensorMap map_ab, const MmaPara
         const int g = ew >> 2;                        // column group: 64 accumulator columns = 32 B-SNPs
         const int a_loc = 16 * q + (lane >> 1);       // A-SNP of this lane inside the CTA's 64
         const int pl = lane & 1;                      // plane held by this lane's TMEM row (0: aa, 1: bb)
-        uint64_t tile_it = 0;
         GW_PROF(long long prof_tw = 0; const long long prof_e0 = clock64();)
-        uint32_t n_sched = 0, I2, J;
-        for (; sched_next_warp(sched, sfull, sempty, lane, n_sched, I2, J); ++tile_it) {
+        uint32_t I2, J;
+        for (uint64_t tile = 0; pipe.next_warp(lane, (uint32_t)tile, I2, J); ++tile) {
             const uint32_t I = 2 * I2 + rank;         // this CTA's 64-SNP A-block
-            const uint32_t buf = (uint32_t)(tile_it & 1);
             const uint64_t gi = (uint64_t)I * MMA_A_SNPS + a_loc;
             // row-role record of this lane's A-SNP. Odd lanes own plane "bb" of A: they see the table with A's
             // genotype labels aa <-> bb exchanged, which the statistic does not depend on, so their record is
@@ -517,10 +436,8 @@ pair_screen_mma_kernel(const __grid_constant__ CUtensorMap map_ab, const MmaPara
                 __syncwarp();
             }
             GW_PROF(const long long w2 = clock64();)
-            if (lane == 0) mbar_wait_wd(&tfull[buf], (uint32_t)((tile_it >> 1) & 1));
-            __syncwarp();
+            const uint32_t buf = pipe.acc_wait(lane, tile);
             GW_PROF(prof_tw += clock64() - w2;)
-            tc_fence_after();
 #pragma unroll 1
             for (int h = 0; h < 2; ++h) {
                 uint32_t v[32];
@@ -599,22 +516,14 @@ pair_screen_mma_kernel(const __grid_constant__ CUtensorMap map_ab, const MmaPara
                     }
                 }
             }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_remote(&tempty[buf], 0);
+            pipe.acc_release(lane, buf);
         }
         GW_PROF(if (p.prof && lane == 0 && (warp == 0 || warp == 15)) {
             unsigned long long *o = p.prof + blockIdx.x * 8;
             o[warp == 0 ? 3 : 7] = (unsigned long long)(clock64() - prof_e0); if (warp == 0) o[4] = (unsigned long long)prof_tw;
         })
     }
-
-    tc_fence_before();
-    cluster_sync_all();                                // neither CTA leaves while its pair may still touch its SM
-    if (warp == MMA_WARP) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-    }
+    pipe.teardown();
 }
 
 // ---- tensor-core roofline probe ---------------------------------------------------------------------
@@ -640,10 +549,7 @@ i8_peak_kernel(uint32_t kblocks, uint32_t seed) {
         reinterpret_cast<uint32_t *>(sm)[q] = w;
     }
     if (tid == 0) { mbar_init(done, 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
+    if (warp == 0) tmem_alloc_pair(tmem_slot);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy stores above -> async-proxy reads of the MMAs
     tc_fence_before();
     __syncthreads();
@@ -666,7 +572,7 @@ i8_peak_kernel(uint32_t kblocks, uint32_t seed) {
     cluster_sync_all();
     if (warp == 0) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+        tmem_dealloc_pair(tmem_base);
     }
 }
 
@@ -798,14 +704,13 @@ static_assert(M4_BLK == TILE, "the four-plane tiles coincide with the 64-SNP mis
 // per eight lanes so that the quads' reads fall on different banks).
 constexpr int M4_XCH_WARP = 1600;
 template <int MODE> struct M4Smem {
-    static constexpr int CPB = MODE == 1 ? 4 : 3;
+    static constexpr int CPB = MODE == 1 ? 4 : 3;                                   // accumulator columns per B-SNP
     static constexpr int KBB = A_STAGE_BYTES + MMA_B_SNPS / 4 * CPB * MMA_KB;       // 32 KiB (split classes) or 28 KiB
-    static constexpr int STG = KPS * KBB;
     static constexpr int XCH = MODE == 1 ? 0 : EPI_WARPS * M4_XCH_WARP;
-    static constexpr size_t BYTES = 1024 + (size_t)MMA_STAGES * STG + XCH + EPI_WARPS * COL_STAGE_BYTES + (2 * MMA_STAGES + 4 + 2 * SCHED_SLOTS) * sizeof(uint64_t) +
-                                    SCHED_SLOTS * sizeof(uint2) + 16;
-    static_assert(KBB % 1024 == 0 && BYTES <= 232448, "stage blocks keep the 1 KiB swizzle alignment; at most 227 KiB per CTA");
 };
+// extra: the exchange rows, then per epilogue warp the PairSide records of its 16 B-SNPs. MODE 2 holds both accumulators per tile.
+template <int MODE>
+using M4Pipe = CtaPipe<MMA_STAGES, KPS, M4Smem<MODE>::KBB, M4Smem<MODE>::XCH + EPI_WARPS * COL_STAGE_BYTES, MODE == 2 ? 1 : 2>;
 
 struct Mma4Params {
     uint32_t TB, NKB, n_bands, band;
@@ -844,120 +749,55 @@ pair_screen_mma4_kernel(const __grid_constant__ CUtensorMap map_ab, const __grid
     constexpr bool SPLIT = MODE == 1, TWOACC = MODE == 2;
     // B side: the padding plane never enters a pair's table, so the missing-call layouts send only three rows per B-SNP to the
     // tensor cores (a 3-D TMA box over the same matrix: sample bytes x 3 of the 4 planes x 32 SNPs = 96 dense rows): N = 192.
-    constexpr int CPB = SPLIT ? 4 : 3;                            // accumulator columns per B-SNP
-    constexpr int B_BYTES = MMA_B_SNPS / 4 * CPB * MMA_KB;        // this CTA's half of B per sample block (32 SNPs)
+    constexpr int CPB = M4Smem<MODE>::CPB;
     constexpr uint32_t IDESC = idesc_i8(M4_BLK * CPB);
-    constexpr int KBB = M4Smem<MODE>::KBB, STG = M4Smem<MODE>::STG;   // bytes per sample block / per stage of this CTA
     extern __shared__ unsigned char smem_raw[];
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    unsigned char *sm = smem_raw + (base - smem_u32(smem_raw));
-    unsigned char *xch_sm = sm + MMA_STAGES * STG;                              // per epilogue warp: product exchange rows (missing-call layouts)
+    M4Pipe<MODE> pipe;
+    unsigned char *xch_sm = pipe.setup(smem_raw);                               // per epilogue warp: product exchange rows (missing-call layouts)
     unsigned char *col_sm = xch_sm + M4Smem<MODE>::XCH;                         // per epilogue warp: PairSide records of its 16 B-SNPs
-    uint64_t *full = reinterpret_cast<uint64_t *>(col_sm + EPI_WARPS * COL_STAGE_BYTES);
-    uint64_t *empty = full + MMA_STAGES;
-    uint64_t *tfull = empty + MMA_STAGES;
-    uint64_t *tempty = tfull + 2;
-    uint64_t *sfull = tempty + 2;                      // tile feed, as in pair_screen_mma_kernel
-    uint64_t *sempty = sfull + SCHED_SLOTS;
-    uint2 *sched = reinterpret_cast<uint2 *>(sempty + SCHED_SLOTS);
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(sched + SCHED_SLOTS);
-
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint32_t rank = cluster_ctarank();
-
-    if (tid == 0) {
-        for (int s = 0; s < MMA_STAGES; ++s) { mbar_init(&full[s], 2); mbar_init(&empty[s], 1); }
-        for (int b = 0; b < 2; ++b) { mbar_init(&tfull[b], 1); mbar_init(&tempty[b], 2 * EPI_WARPS); }
-        for (int b = 0; b < SCHED_SLOTS; ++b) { mbar_init(&sfull[b], 1); mbar_init(&sempty[b], SCHED_CONSUMERS); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == MMA_WARP) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    cluster_sync_all();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
+    const uint32_t rank = pipe.rank;
+    const uint32_t tmem_base = pipe.tmem;
 
     // the tiles this launch computes: the leader's producer skips the others while it draws (TileDraw), the other roles only see these
     auto wanted = [&](uint32_t I2, uint32_t J) -> bool { return TWOACC || ((p.tile_missing[I2] | p.tile_missing[J]) != 0) != SPLIT; };
 
     if (warp == TMA_WARP) {
-        if (lane == 0) {
-            uint64_t it = 0;
-            uint32_t n_sched = 0;
-            TileDraw draw;
-            draw.counter = p.tile_counter; draw.shard = p.shard; draw.n_shards = p.n_shards; draw.TB = p.TB; draw.n_bands = p.n_bands; draw.band = p.band; draw.last = p.n_tiles;
-            for (;;) {
-                uint32_t I2, J;
-                if (rank == 0) {
-                    bool more;
-                    if constexpr (SETS) {
-                        for (;;) {
-                            const uint64_t u = atomicAdd(p.tile_counter, 1ull);
-                            more = u < p.n_tiles;
-                            if (!more) break;
-                            const uint2 e = p.set_tiles[u];
-                            I2 = e.x; J = e.y;
-                            if (wanted(I2, J)) break;
-                        }
-                    } else more = draw.next(I2, J, wanted);
-                    const int slot = (int)(n_sched % SCHED_SLOTS);
-                    mbar_wait_wd(&sempty[slot], ((n_sched / SCHED_SLOTS) & 1u) ^ 1u);
-                    sched_publish(sched, sfull, slot, more ? I2 : SCHED_END, J);
-                    if (!more) break;
-                    ++n_sched;
-                    if constexpr (!SETS) draw.prefetch();
-                } else if (!sched_next(sched, sfull, sempty, n_sched, I2, J)) break;
-                const int a_row = (int)((2 * I2 + rank) * (2 * MMA_A_SNPS)), b_row = (int)(J * MMA_N + rank * MMA_B_SNPS);
-                for (uint32_t kb = 0; kb < p.NKB; kb += KPS, ++it) {
-                    const int st = (int)(it % MMA_STAGES);
-                    const uint32_t nk = min((uint32_t)KPS, p.NKB - kb);
-                    mbar_wait_wd(&empty[st], (uint32_t)(((it / MMA_STAGES) & 1) ^ 1));
-                    unsigned char *dst = sm + st * STG;
-                    if (rank == 0) mbar_expect_tx(&full[st], nk * 2 * (A_STAGE_BYTES + B_BYTES));
-                    else mbar_arrive_remote(&full[st], 0);
-                    for (uint32_t k2 = 0; k2 < nk; ++k2) {
-                        tma_load_2d_pair(dst + k2 * KBB, &map_ab, (int)((kb + k2) * MMA_KB), a_row, &full[st]);
-                        if (SPLIT) tma_load_2d_pair(dst + k2 * KBB + A_STAGE_BYTES, &map_ab, (int)((kb + k2) * MMA_KB), b_row, &full[st]);
-                        else tma_load_3d_pair(dst + k2 * KBB + A_STAGE_BYTES, &map_b3, (int)((kb + k2) * MMA_KB), 0, b_row / M4_PLANES, &full[st]);
-                    }
+        TileDraw td;
+        td.counter = p.tile_counter; td.shard = p.shard; td.n_shards = p.n_shards; td.TB = p.TB; td.n_bands = p.n_bands; td.band = p.band; td.last = p.n_tiles;
+        auto draw = [&](uint32_t &I2, uint32_t &J) -> bool {
+            if constexpr (SETS) {
+                for (;;) {
+                    const uint64_t u = atomicAdd(p.tile_counter, 1ull);
+                    if (u >= p.n_tiles) return false;
+                    const uint2 e = p.set_tiles[u];
+                    I2 = e.x; J = e.y;
+                    if (wanted(I2, J)) return true;
                 }
+            } else {
+                if (!td.next(I2, J, wanted)) return false;
+                td.prefetch();
+                return true;
             }
-        }
+        };
+        auto load = [&](uint32_t I2, uint32_t J, unsigned char *dst, uint32_t blk, uint64_t *full) {
+            const int a_row = (int)((2 * I2 + rank) * (2 * MMA_A_SNPS)), b_row = (int)(J * MMA_N + rank * MMA_B_SNPS);
+            tma_load_2d_pair(dst, &map_ab, (int)(blk * MMA_KB), a_row, full);
+            if (SPLIT) tma_load_2d_pair(dst + A_STAGE_BYTES, &map_ab, (int)(blk * MMA_KB), b_row, full);
+            else tma_load_3d_pair(dst + A_STAGE_BYTES, &map_b3, (int)(blk * MMA_KB), 0, b_row / M4_PLANES, full);
+        };
+        pipe.produce(p.NKB, draw, load);
     } else if (warp == MMA_WARP) {
-        if (lane == 0 && rank == 0) {
-            uint64_t it = 0, tile_it = 0;
-            uint32_t n_sched = 0, I2, J;
-            while (sched_next(sched, sfull, sempty, n_sched, I2, J)) {
-                // two accumulators per tile (TWOACC): buffer 0 = cases, buffer 1 = controls, one tile in flight
-                const uint32_t buf = TWOACC ? 0u : (uint32_t)(tile_it & 1);
-                mbar_wait_wd(&tempty[buf], TWOACC ? (uint32_t)((tile_it & 1) ^ 1) : (uint32_t)(((tile_it >> 1) & 1) ^ 1));
-                tc_fence_after();
-                const uint32_t d_addr = tmem_base + buf * ACC_COLS;
-                for (uint32_t kb = 0; kb < p.NKB; kb += KPS, ++it) {
-                    const int st = (int)(it % MMA_STAGES);
-                    const uint32_t nk = min((uint32_t)KPS, p.NKB - kb);
-                    mbar_wait_wd(&full[st], (uint32_t)((it / MMA_STAGES) & 1));
-                    tc_fence_after();
-                    for (uint32_t k2 = 0; k2 < nk; ++k2) {
-                        const uint32_t a_addr = base + st * STG + k2 * KBB, b_addr = a_addr + A_STAGE_BYTES;
-                        const uint64_t ad = umma_desc(a_addr), bd = umma_desc(b_addr);
-                        const uint32_t blk = kb + k2;                                      // 128-byte sample block of the row
-                        const bool ctrl = TWOACC && blk >= p.case_kb;
-                        const uint32_t d_blk = ctrl ? d_addr + ACC_COLS : d_addr;
-                        const uint32_t first_blk = ctrl ? p.case_kb : 0u;
+        // TWOACC: the case sample blocks accumulate into the tile's accumulator, the control blocks into the next ACC_COLS columns
+        pipe.issue(p.NKB, [&](uint32_t d_addr, uint32_t a_addr, uint32_t blk) {
+            const uint64_t ad = umma_desc(a_addr), bd = umma_desc(a_addr + A_STAGE_BYTES);
+            const bool ctrl = TWOACC && blk >= p.case_kb;
+            const uint32_t d_blk = ctrl ? d_addr + ACC_COLS : d_addr;
+            const uint32_t first_blk = ctrl ? p.case_kb : 0u;
 #pragma unroll
-                        for (int k = 0; k < MMA_KB / UMMA_K; ++k)
-                            tc_mma_i8(d_blk, ad + (uint64_t)(k * UMMA_K >> 4), bd + (uint64_t)(k * UMMA_K >> 4), IDESC, (blk != first_blk) || k != 0);
-                    }
-                    tc_commit_mc(&empty[st], 3);
-                }
-                tc_commit_mc(&tfull[buf], 3);
-                ++tile_it;
-            }
-        }
+            for (int k = 0; k < MMA_KB / UMMA_K; ++k)
+                tc_mma_i8(d_blk, ad + (uint64_t)(k * UMMA_K >> 4), bd + (uint64_t)(k * UMMA_K >> 4), IDESC, (blk != first_blk) || k != 0);
+        });
     } else {
         // ===== epilogue (both CTAs: own 32 A-SNPs x the tile's 64 B-SNPs) =====
         const int ew = warp;
@@ -966,10 +806,8 @@ pair_screen_mma4_kernel(const __grid_constant__ CUtensorMap map_ab, const __grid
         const int a_loc = 8 * q + (lane >> 2);        // A-SNP of this lane inside the CTA's 32
         const uint32_t pl = (uint32_t)lane & 3u;      // plane held by this lane's TMEM row (0 aa, 1 bb, 2 xx, 3 padding)
         const unsigned qbase = (unsigned)lane & ~3u;
-        uint64_t tile_it = 0;
-        uint32_t n_sched = 0, I2, J;
-        while (sched_next_warp(sched, sfull, sempty, lane, n_sched, I2, J)) {
-            const uint32_t buf = TWOACC ? 0u : (uint32_t)(tile_it & 1);
+        uint32_t I2, J;
+        for (uint64_t tile = 0; pipe.next_warp(lane, (uint32_t)tile, I2, J); ++tile) {
             const uint64_t gi = (uint64_t)I2 * M4_BLK + rank * M4_A_SNPS + a_loc;
             // this warp's 16 column-role records (PairSide, 128 bytes each): 2 KiB contiguous -> its shared-memory slot
             unsigned char *my_col = col_sm + ew * COL_STAGE_BYTES;
@@ -982,9 +820,7 @@ pair_screen_mma4_kernel(const __grid_constant__ CUtensorMap map_ab, const __grid
             }
             const PairSide &A = p.side[gi < p.M ? gi : 0];   // read through L1: 8 records per warp, reused for 16 B-SNPs
             const float thr_now = sink_threshold(p.sink);
-            if (lane == 0) mbar_wait_wd(&tfull[buf], TWOACC ? (uint32_t)(tile_it & 1) : (uint32_t)((tile_it >> 1) & 1));
-            __syncwarp();
-            tc_fence_after();
+            const uint32_t buf = pipe.acc_wait(lane, tile);
             // one pair's 3x3x2 table from its products and both SNPs' class counts, then the screen statistic
             auto finish_pair = [&](uint64_t gj, const PairSide &B, const uint32_t (&prod)[CPB][CPB], const uint32_t (&prod_ctl)[3][3]) {
                 uint32_t n[2][3][3];
@@ -1096,19 +932,10 @@ pair_screen_mma4_kernel(const __grid_constant__ CUtensorMap map_ab, const __grid
                     }
                 }
             }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_remote(&tempty[buf], 0);
-            ++tile_it;
+            pipe.acc_release(lane, buf);
         }
     }
-
-    tc_fence_before();
-    cluster_sync_all();
-    if (warp == MMA_WARP) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-    }
+    pipe.teardown();
 }
 
 // operand rows of the four-plane engine: one thread per (SNP, 32-sample word), 32 bytes of each of aa, bb, xx
@@ -1267,19 +1094,6 @@ bool gwasdev_internal_mma_eligible(const gwasdev_store *s) {
     return s->n_case >= 1 && s->n_ctrl >= 1 && s->n_case < (1u << CTRL_SHIFT) && s->n_ctrl < (1u << (31 - CTRL_SHIFT));
 }
 
-static int make_mm_map(gwasdev_store *s, uint32_t box_rows, CUtensorMap *out) {
-    encode_tiled_fn encode = nullptr;
-    { int rc = get_encode_tiled(&encode); if (rc != GWASDEV_OK) return rc; }
-    cuuint64_t gdim[2] = {s->mm_kbytes, s->mm_rows};
-    cuuint64_t gstride[1] = {s->mm_kbytes};
-    cuuint32_t box[2] = {(cuuint32_t)MMA_KB, box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, s->d_mm, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (tensor-core operand matrix) failed (%d)", (int)r); return GWASDEV_ENODEVICE; }
-    return GWASDEV_OK;
-}
-
 // Constants of ksa_upper_bound for a cohort with n_case cases among n samples: the smallest qc (plus a safety
 // factor) with H2(x) >= H2(x0) + H2'(x0)(x - x0) - qc (x - x0)^2 on [0, 1], and q0 = qc x0 n_case + n H2(x0).
 static void bound_constants(uint32_t n_case, uint32_t n, float *qc_out, float *q0_out) {
@@ -1316,7 +1130,7 @@ static int ensure_mma_inputs(gwasdev_store *s) {
         GW_LAUNCHED();
         if (!s->tmap_mm && posix_memalign(&s->tmap_mm, 64, sizeof(CUtensorMap)) != 0) { s->tmap_mm = nullptr; set_error("out of host memory"); return GWASDEV_ENOMEM; }
         int rc;
-        if ((rc = make_mm_map(s, 2 * MMA_A_SNPS, (CUtensorMap *)s->tmap_mm)) != GWASDEV_OK) return rc;   // 128-row boxes: a CTA's A rows / its half of B
+        if ((rc = encode_operand_map(s->d_mm, s->mm_rows, s->mm_kbytes, 2 * MMA_A_SNPS, (CUtensorMap *)s->tmap_mm)) != GWASDEV_OK) return rc;   // 128-row boxes: a CTA's A rows / its half of B
         // schedule: bands of as many A-blocks as fit 32 MB of operand rows, the last band possibly shorter
         const uint32_t TB = (uint32_t)(Msnp / MMA_BLK);
         s->mm_band = schedule_band((uint64_t)MMA_N * s->mm_kbytes);
@@ -1396,33 +1210,25 @@ uint64_t gwasdev_internal_mma_shard_pairs(const gwasdev_store *s, uint32_t shard
     return pairs;
 }
 
-static size_t mma_smem_bytes() {
-    return 1024 + (size_t)MMA_STAGES * STAGE_BYTES_MMA + EPI_WARPS * COL_STAGE_BYTES + (2 * MMA_STAGES + 4 + 2 * SCHED_SLOTS) * sizeof(uint64_t) + SCHED_SLOTS * sizeof(uint2) + 16;
-}
-
 template <bool SETS = false>
 static int launch_mma(gwasdev_store *s, MmaParams &p, uint64_t my_tiles) {
-    int sms = 0;
-    GW_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
-    const size_t smem = mma_smem_bytes();
-    GW_CUDA(cudaFuncSetAttribute(pair_screen_mma_kernel<SETS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const unsigned pairs = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)sms / 2, my_tiles));   // one CTA pair per TPC
 #ifdef GWASDEV_SWEEP
     const bool prof = getenv("GWASDEV_MMA_PROF") != nullptr && !p.dump;
 #else
     const bool prof = false;
 #endif
     unsigned long long *d_prof = nullptr;
-    if (prof) {
-        GW_CUDA(cudaMalloc(&d_prof, (size_t)2 * pairs * 8 * sizeof(unsigned long long)));
-        GW_CUDA(cudaMemsetAsync(d_prof, 0, (size_t)2 * pairs * 8 * sizeof(unsigned long long), s->stream));
+    if (prof) {   // 8 timers per CTA; launch_cta_pairs runs at most one CTA per SM
+        int sms = 0;
+        GW_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
+        GW_CUDA(cudaMalloc(&d_prof, (size_t)sms * 8 * sizeof(unsigned long long)));
+        GW_CUDA(cudaMemsetAsync(d_prof, 0, (size_t)sms * 8 * sizeof(unsigned long long), s->stream));
     }
     p.prof = d_prof;
-    if (!s->d_tile_counter) GW_CUDA(cudaMalloc(&s->d_tile_counter, sizeof(unsigned long long)));
-    GW_CUDA(cudaMemsetAsync(s->d_tile_counter, 0, sizeof(unsigned long long), s->stream));
-    p.tile_counter = s->d_tile_counter;
-    pair_screen_mma_kernel<SETS><<<2 * pairs, MMA_THREADS, smem, s->stream>>>(*(const CUtensorMap *)s->tmap_mm, p);
-    GW_LAUNCHED();
+    unsigned pairs = 0;
+    { const int rc = launch_cta_pairs(s, pair_screen_mma_kernel<SETS>, MmaPipe::SMEM, my_tiles, p, &pairs, nullptr,
+                                         *(const CUtensorMap *)s->tmap_mm);
+      if (rc != GWASDEV_OK) return rc; }
     if (prof) {
         std::vector<unsigned long long> h((size_t)2 * pairs * 8);
         GW_CUDA(cudaMemcpyAsync(h.data(), d_prof, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
@@ -1486,22 +1292,16 @@ static int ensure_mma4_inputs(gwasdev_store *s, int mode) {
     }
     GW_LAUNCHED();
     if (!s->tmap_mm4 && posix_memalign(&s->tmap_mm4, 64, 2 * sizeof(CUtensorMap)) != 0) { s->tmap_mm4 = nullptr; set_error("out of host memory"); return GWASDEV_ENOMEM; }
-    encode_tiled_fn encode = nullptr;
-    { int rc = get_encode_tiled(&encode); if (rc != GWASDEV_OK) return rc; }
-    cuuint64_t gdim[2] = {s->mm4_kbytes, s->mm4_rows};
-    cuuint64_t gstride[1] = {s->mm4_kbytes};
-    cuuint32_t box[2] = {(cuuint32_t)MMA_KB, (cuuint32_t)(2 * MMA_A_SNPS)};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = encode((CUtensorMap *)s->tmap_mm4, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, s->d_mm4, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (four-plane operand matrix) failed (%d)", (int)r); return GWASDEV_ENODEVICE; }
+    { const int rc = encode_operand_map(s->d_mm4, s->mm4_rows, s->mm4_kbytes, 2 * MMA_A_SNPS, (CUtensorMap *)s->tmap_mm4); if (rc != GWASDEV_OK) return rc; }
     {   // the B side of the missing-call layouts: planes 0..2 of 32 SNPs as one dense 96-row box
+        encode_tiled_fn encode = nullptr;
+        { const int rc = get_encode_tiled(&encode); if (rc != GWASDEV_OK) return rc; }
         cuuint64_t gdim3[3] = {s->mm4_kbytes, (cuuint64_t)M4_PLANES, s->mm4_rows / M4_PLANES};
         cuuint64_t gstride3[2] = {s->mm4_kbytes, (cuuint64_t)M4_PLANES * s->mm4_kbytes};
         cuuint32_t box3[3] = {(cuuint32_t)MMA_KB, 3, (cuuint32_t)(MMA_B_SNPS / 4)};
         cuuint32_t estr3[3] = {1, 1, 1};
-        r = encode((CUtensorMap *)s->tmap_mm4 + 1, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, s->d_mm4, gdim3, gstride3, box3, estr3, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        const CUresult r = encode((CUtensorMap *)s->tmap_mm4 + 1, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, s->d_mm4, gdim3, gstride3, box3, estr3, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (three-plane B box) failed (%d)", (int)r); return GWASDEV_ENODEVICE; }
     }
     s->mm4_band = m4_band(s, mode);
@@ -1606,23 +1406,11 @@ int gwasdev_internal_screen_mma4(gwasdev_store *s, const CandSink &sink, uint32_
     if (set) { p.n_tiles = set->n_tiles; p.shard = 0; p.n_shards = 1; p.set_tiles = set->tiles; p.set_c1 = set->c1; p.set_a1 = set->a1; }
     const uint64_t my_tiles = shard_tiles_before(p.n_tiles, p.shard, p.n_shards);
     if (my_tiles == 0) return GWASDEV_OK;
-    int sms = 0;
-    GW_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
-    const unsigned pairs = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)sms / 2, my_tiles));
-    if (!s->d_tile_counter) GW_CUDA(cudaMalloc(&s->d_tile_counter, sizeof(unsigned long long)));
-    GW_CUDA(cudaMemsetAsync(s->d_tile_counter, 0, sizeof(unsigned long long), s->stream));
-    p.tile_counter = s->d_tile_counter;
-#define SCREEN4(MODE_, SETS_)                                                                                                  \
-    do {                                                                                                                       \
-        const size_t smem = M4Smem<MODE_>::BYTES;                                                                              \
-        GW_CUDA(cudaFuncSetAttribute(pair_screen_mma4_kernel<MODE_, SETS_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        pair_screen_mma4_kernel<MODE_, SETS_><<<2 * pairs, MMA_THREADS, smem, s->stream>>>(((const CUtensorMap *)s->tmap_mm4)[0], ((const CUtensorMap *)s->tmap_mm4)[1], p); \
-    } while (0)
-    if (set) { if (mode == 1) SCREEN4(1, true); else if (mode == 2) SCREEN4(2, true); else SCREEN4(0, true); }
-    else if (mode == 1) SCREEN4(1, false); else if (mode == 2) SCREEN4(2, false); else SCREEN4(0, false);
+    const CUtensorMap *maps = (const CUtensorMap *)s->tmap_mm4;
+#define SCREEN4(MODE_, SETS_) launch_cta_pairs(s, pair_screen_mma4_kernel<MODE_, SETS_>, M4Pipe<MODE_>::SMEM, my_tiles, p, nullptr, nullptr, maps[0], maps[1])
+    if (set) return mode == 1 ? SCREEN4(1, true) : mode == 2 ? SCREEN4(2, true) : SCREEN4(0, true);
+    return mode == 1 ? SCREEN4(1, false) : mode == 2 ? SCREEN4(2, false) : SCREEN4(0, false);
 #undef SCREEN4
-    GW_LAUNCHED();
-    return GWASDEV_OK;
 }
 
 // operands and records of the two kernels ahead of a set screen's timed region

@@ -12,7 +12,7 @@
 // (GWASDEV_OPT_PERM_OPERAND_BYTES) and is dropped when rows change; above the budget it is expanded one SNP chunk at a time.
 // The A operand (a few MB) is rebuilt by every call.
 //
-// Kernel (perm_gemm_kernel, permute_gemm.cuh, compiled in marginal.cu): the pair screens' CTA-pair pipeline (mma_common.cuh). Tiles are (256 permutations: 128 TMEM lanes per CTA) x
+// Kernel (perm_gemm_kernel, permute_gemm.cuh, compiled in marginal.cu): the CTA-pair pipeline of mma_common.cuh. Tiles are (256 permutations: 128 TMEM lanes per CTA) x
 // (64 SNPs: each CTA stages 32 SNPs of B), taken from a device counter in SNP-major order, so the tiles in flight share a few
 // SNP blocks and B is read from DRAM about once per call. One TMEM lane holds one permutation, so a thread owns every plane of
 // its (permutation, SNP) elements: the statistics come from the marginal scan's own chi2_tests (bit-identical), the per-permutation
@@ -112,19 +112,6 @@ static double chisq_q(double x, int df) { return x > 0.0 ? (df == 1 ? std::erfc(
 
 using namespace gwasdev;
 
-int gwasdev::encode_operand_map(void *ptr, uint64_t rows, uint32_t kbytes, uint32_t box_rows, CUtensorMap *out) {
-    encode_tiled_fn encode = nullptr;
-    { const int rc = get_encode_tiled(&encode); if (rc != GWASDEV_OK) return rc; }
-    cuuint64_t gdim[2] = {kbytes, rows};
-    cuuint64_t gstride[1] = {kbytes};
-    cuuint32_t box[2] = {(cuuint32_t)MMA_KB, box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    const CUresult r = encode(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, ptr, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (operand rows) failed (%d)", (int)r); return GWASDEV_ENODEVICE; }
-    return GWASDEV_OK;
-}
-
 // planes of SNPs [snp0, snp0 + n) into d_pb (rows from 0)
 static int build_planes(gwasdev_store *s, int PL, uint64_t snp0, uint64_t n) {
     const uint32_t kbytes = 32 * s->Wr;
@@ -147,19 +134,12 @@ static int launch_perm(gwasdev_store *s, int PL, PermParams p, uint64_t pa_rows,
     if ((rc = encode_operand_map(s->d_pb, (uint64_t)PL * pb_snps, kbytes, PSNP_HALF * PL, &maps[1])) != GWASDEV_OK) return rc;
     p.NKB = kbytes / MMA_KB;
     p.n_tiles = (uint64_t)p.n_pblk * ((p.nsnp + PSNP_BLK - 1) / PSNP_BLK);
-    int sms = 0;
-    GW_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, s->device));
-    const unsigned pairs = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)sms / 2, p.n_tiles));
-    if (!s->d_tile_counter) GW_CUDA(cudaMalloc(&s->d_tile_counter, sizeof(unsigned long long)));
-    GW_CUDA(cudaMemsetAsync(s->d_tile_counter, 0, sizeof(unsigned long long), s->stream));
-    p.tile_counter = s->d_tile_counter;
     cudaEvent_t e0, e1;
     GW_CUDA(cudaEventCreate(&e0));
     evs.push_back(e0);
     GW_CUDA(cudaEventCreate(&e1));
     evs.push_back(e1);
-    GW_CUDA(cudaEventRecord(e0, s->stream));
-    { const int rc = gwasdev_internal_perm_gemm(s, PL, p, maps, pairs); if (rc != GWASDEV_OK) return rc; }
+    { const int rc = gwasdev_internal_perm_gemm(s, PL, p, maps, e0); if (rc != GWASDEV_OK) return rc; }
     GW_CUDA(cudaEventRecord(e1, s->stream));
     return GWASDEV_OK;
 }

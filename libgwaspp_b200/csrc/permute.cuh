@@ -26,7 +26,8 @@ struct PermParams {
     unsigned long long *tile_counter;  // zero at launch
 };
 
-// launches perm_gemm_kernel<PL> on `pairs` CTA pairs over the A / B tensor maps maps[0], maps[1] (marginal.cu)
-int gwasdev_internal_perm_gemm(gwasdev_store *s, int PL, const PermParams &p, const CUtensorMap *maps, unsigned pairs);
+// launches perm_gemm_kernel<PL> over p.n_tiles tiles and the A / B tensor maps maps[0], maps[1], recording `start` right
+// before the kernel (marginal.cu)
+int gwasdev_internal_perm_gemm(gwasdev_store *s, int PL, PermParams &p, const CUtensorMap *maps, cudaEvent_t start);
 
 }  // namespace gwasdev
